@@ -25,6 +25,9 @@ ONE JSON line.  See DESIGN.md "Measurement" for how every field is derived.
 
 --impl reference runs only that CPU path and prints the same line shape with "impl": "reference".
 --cfg1 measures BASELINE.json configs[0] instead (the cvsteer-run per-file body on the bundled test image).
+--dump-outputs DIR writes, after the K timed steps, what the last one computed: DIR/<plane>.npy (float32) for every output plane
+of the headline launch, each at the same 2^20 pixels of the 64-frame batch (flat indices drawn by np.random.default_rng(0),
+sorted).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -47,6 +50,7 @@ MODES = {
 }
 FP32_NOMINAL = 148 * 128 * 1.965e9           # fp32 instructions/s: 148 SMs x 128 lanes x max SM clock
 PYR5 = sum(0.25 ** l for l in range(5))      # pixels of a 5-level pyramid per level-0 pixel (1.332)
+DUMP_PIXELS = 1 << 20                        # --dump-outputs: sampled pixels per plane (12 planes at most: 48 MB in all)
 
 
 def env_int(k, d):
@@ -303,6 +307,7 @@ def run_headline(cx, args):
     launches = lib.cvs_launch_count() - l0
     launch = g.last_launch()
     value = cx.world * px / 1e6 / (ms / 1e3)
+    dump = output_sample(cx, outs, planes) if args.dump_outputs and cx.rank == 0 else None
 
     # sustained: the same launch back to back for >= 2 s (the power cap pulls the SM clock down after a few hundred ms)
     sustained = None
@@ -319,7 +324,25 @@ def run_headline(cx, args):
            "l2": "inputs (531 MB/GPU) larger than the 126 MB L2; no flush needed",
            "grid": launch["grid"], "block": launch["block"], "smem": launch["smem"]}
     return dict(value=value, ms=ms, clocks=clocks, launches=int(launches), roofline=roof, config=cfg,
-                state=(g, x, outs, mask, planes, px))
+                state=(g, x, outs, mask, planes, px), dump=dump)
+
+
+def output_sample(cx, outs, planes):
+    """The headline planes as they are now (after the last timed step) at DUMP_PIXELS fixed, seeded positions of the batch."""
+    import numpy as np
+    from cvsteer_b200 import capi
+    px = FRAMES * ROWS * COLS
+    idx = np.sort(np.random.default_rng(0).choice(px, min(px, DUMP_PIXELS), replace=False))
+    assert idx.size * 4 * len(planes) <= 64 << 20
+    idx = cx.torch.from_numpy(idx).to(cx.dev)
+    return {capi.G2_PLANE_NAMES[p]: outs[p].view(-1)[idx].cpu().numpy() for p in planes}
+
+
+def write_dump(d, arrays):
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(a, np.float32))
 
 
 def run_e2e(cx, args, state):
@@ -524,6 +547,9 @@ def run_ours(args, rank, local_rank, world):
         cx.fp32_measured = None
 
     head = run_headline(cx, args)
+    dump = head.pop("dump")
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     e2e = None if args.no_e2e else run_e2e(cx, args, head["state"])
     head.pop("state")
     torch.cuda.empty_cache()
@@ -625,7 +651,13 @@ def main():
     ap.add_argument("--frames-total", type=int, default=256, help="cfg3 / cfg4: frames in total over all GPUs")
     ap.add_argument("--big", type=int, default=32768, help="cfg5: side of the single large image")
     ap.add_argument("--cfg1", action="store_true", help="configs[0] instead: cvsteer-run per-file body on the bundled test image")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of what the last one "
+                                                          "computed to DIR/<plane>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.cfg1 or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if args.cfg1:
         if rank == 0:

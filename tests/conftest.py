@@ -21,8 +21,22 @@ def fish_fixture():
 
 
 @pytest.fixture(scope="session")
-def fish_oracle():
-    return dict(np.load(os.path.join(GOLDEN, "fish_oracle_cv2_4_13.npz")))
+def fish_oracle_golden():
+    """Per plane of the oracle on the fish image: shape, SHA-256 and a seeded sample of the committed cv2 4.13.0 vectors."""
+    import json
+    with open(os.path.join(GOLDEN, "fish_oracle_cv2_4_13.json")) as f:
+        return json.load(f)["planes"]
+
+
+@pytest.fixture(scope="session")
+def fish_oracle(fish_fixture, fish_oracle_golden):
+    """The committed cv2 4.13.0 vectors in full: rebuilt by the oracle and checked bit for bit against their digests."""
+    from tests import util
+    planes = util.fish_oracle_planes(fish_fixture["fish"])
+    assert sorted(planes) == sorted(fish_oracle_golden)
+    for k, v in planes.items():
+        util.assert_matches_golden(k, v, fish_oracle_golden[k])
+    return planes
 
 
 @pytest.fixture(scope="session")

@@ -1,18 +1,24 @@
-"""Generate tests/golden/*.npz from the reference's own test fixtures.
+"""Generate tests/golden/* from the reference's own test fixtures.
 
-Run HERE (the build container), where /root/reference exists; the GPU box never reads
-/root/reference, it only loads the committed .npz files.
+    python tests/golden/make_golden.py [--reference <headupinclouds/cvsteer checkout>]
 
-Inputs (read-only, reference test/test.cpp:41-44):
+With --reference, fish_fixture.npz is rebuilt from the reference's test data (read-only,
+reference test/test.cpp:41-44):
     test/Pterois_volitans_Manado-e_edit_smallest.h   input JPEG (256x185 gray)
     test/edges.h, test/linesDark.h, test/linesBright.h   expected-output JPEGs
 The `xxd -i` byte arrays are parsed as text, the JPEG bytes decoded with cv2
 (IMREAD_GRAYSCALE, as test/test.cpp:53-56 does) and the DECODED PIXELS are stored,
-so the fixtures do not depend on the libjpeg build of whichever box runs the tests.
+so the fixtures do not depend on the libjpeg build of whichever machine runs the tests.
+Without it, the committed fish_fixture.npz is used.
 
-Also stores float-level oracle outputs on the fish image (cv2 4.13.0) as regression
-vectors for the oracle itself and as GPU parity fixtures.
+Then the float-level oracle outputs on the fish image (cv2 4.13.0) are recorded in
+fish_oracle_cv2_4_13.json as regression vectors for the oracle itself and as GPU parity
+fixtures: per plane its shape, the SHA-256 of its float32 bytes and the values at 32 seeded
+positions (the planes themselves, 6.5 MB, are rebuilt by the oracle at test time and checked
+against these bit for bit); and the default taps in taps_default.npz.
 """
+import argparse
+import json
 import os
 import re
 import sys
@@ -23,8 +29,9 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import cvsteer_ref as ref  # noqa: E402
+from tests.util import fish_oracle_planes, plane_digest  # noqa: E402
 
-REF = "/root/reference/test"
+SAMPLES = 32
 
 
 def read_xxd(path):
@@ -41,30 +48,38 @@ def decode(path):
     return img
 
 
-def main():
-    fish = decode(f"{REF}/Pterois_volitans_Manado-e_edit_smallest.h")
-    edges = decode(f"{REF}/edges.h")
-    dark = decode(f"{REF}/linesDark.h")
-    bright = decode(f"{REF}/linesBright.h")
+def write_fixture(reference):
+    t = os.path.join(reference, "test")
+    fish = decode(f"{t}/Pterois_volitans_Manado-e_edit_smallest.h")
+    edges = decode(f"{t}/edges.h")
+    dark = decode(f"{t}/linesDark.h")
+    bright = decode(f"{t}/linesBright.h")
     assert fish.shape == (185, 256) and int(fish.sum()) == 6968201, (fish.shape, fish.sum())
     np.savez_compressed(os.path.join(HERE, "fish_fixture.npz"), fish=fish, edges_gt=edges,
                         lines_dark_gt=dark, lines_bright_gt=bright)
 
-    # float-level oracle outputs (cv2 4.13.0) on the fish image
-    f2, (g2, h2, e, mag, phase) = ref.g2_full(fish)
-    out = {k: getattr(f2, k) for k in ref.SteerableFiltersG2.PLANES}
-    out.update(c1=f2.c1, c2=f2.c2, c3=f2.c3, theta=f2.theta, strength=f2.strength,
-               g2=g2, h2=h2, e=e, magnitude=mag, phase=phase)
-    f4 = ref.SteerableFiltersG4(fish)
-    out.update({k: getattr(f4, k) for k in ref.SteerableFiltersG4.PLANES})
-    g4s, h4s = f4.steer_scalar(0.3)
-    g4m, h4m, mag4, ph4 = f4.steer_map_full(f2.theta)
-    out.update(g4_s03=g4s, h4_s03=h4s, g4_map=g4m, h4_map=h4m, mag4=mag4, phase4=ph4)
-    lv = ref.pyramid(fish, 5)
-    for i, l in enumerate(lv[1:], 1):
-        out[f"pyr{i}"] = l
-    out = {k: np.ascontiguousarray(v, np.float32) for k, v in out.items()}
-    np.savez_compressed(os.path.join(HERE, "fish_oracle_cv2_4_13.npz"), **out)
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--reference", help="headupinclouds/cvsteer checkout: rebuild fish_fixture.npz from its test data")
+    a = ap.parse_args()
+    if a.reference:
+        write_fixture(a.reference)
+    fish = np.load(os.path.join(HERE, "fish_fixture.npz"))["fish"]
+
+    # float-level oracle outputs (cv2 4.13.0) on the fish image: digest + seeded sample per plane, one plane per line
+    out = {k: np.ascontiguousarray(v, np.float32) for k, v in fish_oracle_planes(fish).items()}
+    lines = []
+    for k, v in out.items():
+        idx = np.sort(np.random.default_rng(0).choice(v.size, min(SAMPLES, v.size), replace=False))
+        entry = {"shape": list(v.shape), "sha256": plane_digest(v), "sample_index": [int(i) for i in idx],
+                 "sample": [float(x) for x in v.reshape(-1)[idx]]}
+        lines.append(f"  {json.dumps(k)}: {json.dumps(entry)}")
+    with open(os.path.join(HERE, "fish_oracle_cv2_4_13.json"), "w") as f:
+        f.write('{"cv2": %s,\n "input": "fish_fixture.npz fish (uint8 185x256), width 4 spacing 0.67 (G2/H2), '
+                'width 6 spacing 0.5 (G4/H4)",\n "planes": {\n%s\n }\n}\n' % (json.dumps(cv2.__version__), ",\n".join(lines)))
+
+    f2, f4 = ref.SteerableFiltersG2(fish), ref.SteerableFiltersG4(fish)
     taps = {n: getattr(f2, n)[0] for n in ("g1", "g2", "g3", "h1", "h2", "h3", "h4")}
     taps.update({"G4_" + n: getattr(f4, n)[0] for n in
                  ("g1", "g2", "g3", "g4", "g5", "h1", "h2", "h3", "h4", "h5", "h6")})

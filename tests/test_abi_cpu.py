@@ -90,23 +90,34 @@ def test_header_is_plain_c_and_c_caller_runs():
 
 def test_band_contract_is_validated_before_any_cuda_call():
     """Band mode: the buffer must hold the footprint of the requested output rows; a short halo is an argument error
-    (it would silently filter zeros), reported before the library touches CUDA."""
+    (it would silently filter zeros), reported before the library touches CUDA.  An accepted geometry then runs on the
+    device (device buffers) or, without one, reaches the no-device error (host buffers: nothing is launched)."""
     import ctypes as C
+
+    import torch
 
     from cvsteer_b200 import capi
     lib = capi.lib()
-    buf, out = (C.c_float * (40 * 16))(), (C.c_float * (50 * 8))()
+    device = torch.cuda.is_available()
+    if device:
+        keep = torch.zeros(40 * 16, device="cuda:0"), torch.zeros(50 * 8, device="cuda:0")
+        buf, out = keep[0].data_ptr(), keep[1].data_ptr()
+    else:
+        keep = (C.c_float * (40 * 16))(), (C.c_float * (50 * 8))()
+        buf, out = C.addressof(keep[0]), C.addressof(keep[1])
     b = capi.Batch()
-    b.in_, b.in_is_u8, b.n, b.rows, b.cols = C.addressof(buf), 0, 1, 40, 16
+    b.in_, b.in_is_u8, b.n, b.rows, b.cols = buf, 0, 1, 40, 16
     b.in_pitch, b.in_frame_stride, b.out_pitch, b.out_frame_stride = 64, 64 * 40, 32, 32 * 50
     b.full_rows, b.y_origin, b.out_row_origin = 100, 10, 6                    # buffer = image rows [10, 50)
     for begin, end, ok in ((6, 20, True), (5, 20, False), (6, 26, False), (6, 24, True), (20, 20, False)):
         b.out_row_begin, b.out_row_end = begin, end                          # pyr_down rows y read input rows 2y-2 .. 2y+2
         rc = lib.cvs_pyr_down_dev(0, C.byref(b), out, None)
         if ok:
-            assert rc != capi.ERR_INVALID_ARG, lib.cvs_last_error()          # geometry accepted (then CUDA, absent here)
+            assert rc == (capi.OK if device else capi.ERR_CUDA), lib.cvs_last_error()   # geometry accepted
         else:
             assert rc == capi.ERR_INVALID_ARG and (b"need" in lib.cvs_last_error() or b"invalid" in lib.cvs_last_error())
+    if device:
+        torch.cuda.synchronize()
 
 
 def test_band_context_arguments_and_no_device():

@@ -22,6 +22,12 @@ def test_reference_arm_json_contract():
     assert "workload" in line["config"]
 
 
+def test_dump_outputs_is_for_the_gpu_path(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
+                        "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "out").exists()
+
+
 def test_reference_arm_nonzero_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],

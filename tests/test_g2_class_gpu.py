@@ -44,7 +44,7 @@ def _check_steer(got, o, theta, rng, name=""):
 
 
 def test_fish_matches_golden_vectors(fish_fixture, fish_oracle):
-    """Committed cv2-4.13.0 vectors: no oracle import needed for this comparison."""
+    """Committed cv2-4.13.0 vectors (rebuilt by the oracle and checked bit for bit against their digests)."""
     fish = fish_fixture["fish"]
     f = cb.SteerableFiltersG2(fish, 4, 0.67)  # uint8 in, like the reference callers
     rng = basis_range([fish_oracle[k] for k in STATE])

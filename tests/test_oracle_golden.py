@@ -5,6 +5,7 @@ import numpy as np
 import pytest
 
 from oracle import cvsteer_ref as ref
+from tests.util import assert_matches_golden
 
 
 def _recode(x):
@@ -97,16 +98,16 @@ def test_known_taps():
             assert np.array_equal(k, -k[::-1] if odd else k[::-1])
 
 
-def test_golden_vectors_match_oracle(fish_fixture, fish_oracle):
+def test_golden_vectors_match_oracle(fish_fixture, fish_oracle_golden):
     """The committed float-level vectors are what the oracle produces today (same cv2)."""
     if cv2.__version__ != "4.13.0":
         pytest.skip("vectors were generated with cv2 4.13.0")
     fish = fish_fixture["fish"]
     f2, (g2, h2, e, mag, phase) = ref.g2_full(fish)
     for k in ref.SteerableFiltersG2.PLANES + ("c1", "c2", "c3", "theta", "strength"):
-        assert np.array_equal(getattr(f2, k), fish_oracle[k]), k
-    assert np.array_equal(phase, fish_oracle["phase"])
-    assert np.array_equal(mag, fish_oracle["magnitude"])
+        assert_matches_golden(k, getattr(f2, k), fish_oracle_golden[k])
+    assert_matches_golden("phase", phase, fish_oracle_golden["phase"])
+    assert_matches_golden("magnitude", mag, fish_oracle_golden["magnitude"])
 
 
 def test_wrap_and_phase_weights():
@@ -136,16 +137,16 @@ def test_pyr_down_definition():
     np.testing.assert_allclose(out, full[::2, ::2], atol=1e-4)
 
 
-def test_live_oracle_reproduces_committed_g2_vectors_bitwise(fish_fixture, fish_oracle):
-    """The G2/H2 vectors in tests/golden/fish_oracle_cv2_4_13.npz were written by tests/golden/make_golden.py with the literal
-    float64 `double * Mat1f` round trip and the fancy-index `copyTo`; the oracle now uses a float32 multiply for the dyadic
-    coefficients of G2.cpp:93-95 and np.copyto -- this pins that both are bit-identical to what was committed."""
+def test_live_oracle_reproduces_committed_g2_vectors_bitwise(fish_fixture, fish_oracle_golden):
+    """The G2/H2 vectors digested in tests/golden/fish_oracle_cv2_4_13.json were first written by tests/golden/make_golden.py
+    with the literal float64 `double * Mat1f` round trip and the fancy-index `copyTo`; the oracle now uses a float32 multiply
+    for the dyadic coefficients of G2.cpp:93-95 and np.copyto -- this pins that both are bit-identical to what was committed."""
     f, (g2, h2, e, mag, phase) = ref.g2_full(fish_fixture["fish"], 4, 0.67)
     live = dict(c1=f.c1, c2=f.c2, c3=f.c3, theta=f.theta, strength=f.strength, g2=g2, h2=h2, e=e, magnitude=mag, phase=phase)
     for k in ref.SteerableFiltersG2.PLANES:
         live[k] = getattr(f, k)
     for k, v in live.items():
-        assert v.dtype == np.float32 and np.array_equal(v, fish_oracle[k]), k
+        assert_matches_golden(k, v, fish_oracle_golden[k])
     # ... and the coefficient shortcut itself, including values the fish image does not reach
     m = (np.random.default_rng(5).standard_normal((64, 64)) * 1e4).astype(np.float32)
     m[0, :6] = [0.0, 1e-45, -1e-45, 3e38, 1e-38, -2e-38]
