@@ -51,6 +51,25 @@ def _batch_struct(x: torch.Tensor, out_pitch: int, out_frame_stride: int, band: 
     return b
 
 
+# output plane dtype -> cvs_out_format: 16-bit planes are the fp32 planes rounded to nearest even (include/cvsteer_c.h)
+_OUT_FORMATS = {torch.float32: capi.OUT_F32, torch.float16: capi.OUT_F16, torch.bfloat16: capi.OUT_BF16}
+
+
+def _out_format(dtype) -> int:
+    if dtype not in _OUT_FORMATS:
+        raise capi.CvsError(capi.ERR_INVALID_ARG, f"output planes are float32, float16 or bfloat16, not {dtype}")
+    return _OUT_FORMATS[dtype]
+
+
+def _host_format(outs_host: Dict[int, torch.Tensor]):
+    """(cvs_out_format, element size) of the pinned output planes of one run_host call: they share one dtype."""
+    dtypes = {t.dtype for t in outs_host.values()}
+    if len(dtypes) != 1:
+        raise capi.CvsError(capi.ERR_INVALID_ARG, f"the output planes of one call share one dtype, got {sorted(map(str, dtypes))}")
+    dt = dtypes.pop()
+    return _out_format(dt), torch.empty((), dtype=dt).element_size()
+
+
 def _stream_ptr(stream):
     s = stream if stream is not None else torch.cuda.current_stream()
     return C.c_void_p(s.cuda_stream)
@@ -79,10 +98,13 @@ class _FusedBatch:
 
     def run(self, frames: torch.Tensor, mask: int, steer: int = capi.STEER_DOMINANT, theta: float = 0.0,
             theta_map: Optional[torch.Tensor] = None, outs: Optional[Dict[int, torch.Tensor]] = None,
-            band: Optional[Band] = None, stream=None, next_level: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+            band: Optional[Band] = None, stream=None, next_level: Optional[torch.Tensor] = None,
+            out_dtype: torch.dtype = torch.float32) -> Dict[str, torch.Tensor]:
         """One fused launch over the whole batch.  Returns {plane name: tensor [n, out_rows, cols]}.
         next_level: optional contiguous float32 [n, (rows+1)//2, (cols+1)//2]; the same launch fills it with
-        cv::pyrDown(frames) from the tile it stages anyway (whole frames only)."""
+        cv::pyrDown(frames) from the tile it stages anyway (whole frames only).
+        out_dtype: float32, or float16 / bfloat16 planes that are the float32 planes rounded to nearest even (theta_map and
+        next_level stay float32)."""
         x = _as_batch(frames)
         if x.device.index != self.device:
             raise capi.CvsError(capi.ERR_INVALID_ARG, f"frames live on cuda:{x.device.index}, this handle on cuda:{self.device}")
@@ -90,13 +112,15 @@ class _FusedBatch:
         out_rows = rows if band is None else band.row_end - band.row_begin
         nplanes = len(self._names)
         planes = [p for p in range(nplanes) if mask >> p & 1]
+        fmt = _out_format(out_dtype)
+        es = 4 if fmt == capi.OUT_F32 else 2
         if outs is None:
-            outs = {p: torch.empty((n, out_rows, cols), dtype=torch.float32, device=x.device) for p in planes}
+            outs = {p: torch.empty((n, out_rows, cols), dtype=out_dtype, device=x.device) for p in planes}
         arr = (C.c_void_p * nplanes)()
         for p in planes:
             t = outs[p]
-            if t.shape != (n, out_rows, cols) or t.dtype != torch.float32 or not t.is_contiguous() or not t.is_cuda:
-                raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"output plane {p}: need contiguous CUDA float32 {(n, out_rows, cols)}")
+            if t.shape != (n, out_rows, cols) or t.dtype != out_dtype or not t.is_contiguous() or not t.is_cuda:
+                raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"output plane {p}: need contiguous CUDA {out_dtype} {(n, out_rows, cols)}")
             arr[p] = t.data_ptr()
         tm = None
         if steer == capi.STEER_MAP:
@@ -108,21 +132,26 @@ class _FusedBatch:
                 raise capi.CvsError(capi.ERR_SIZE_MISMATCH,
                                     f"theta_map must be a contiguous float32 tensor {(n, out_rows, cols)} on {x.device}")
             tm = C.c_void_p(theta_map.data_ptr())
-        b = _batch_struct(x, cols * 4, out_rows * cols * 4, band)
+        b = _batch_struct(x, cols * es, out_rows * cols * es, band)
         if next_level is not None:
             want = (n, (rows + 1) // 2, (cols + 1) // 2)
             if tuple(next_level.shape) != want or next_level.dtype != torch.float32 or not next_level.is_contiguous():
                 raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"next_level must be contiguous float32 {want}")
             b.next_level = next_level.data_ptr()
             b.next_pitch, b.next_frame_stride = want[2] * 4, want[1] * want[2] * 4
-        fn = getattr(self._lib, f"cvs_{self._prefix}_run_batch_dev")
         with torch.cuda.device(self.device):   # the C call makes the handle's GPU current; torch's current device is restored
-            capi.check(fn(self._h, C.byref(b), mask, steer, theta, tm, arr, _stream_ptr(stream)))
+            if fmt == capi.OUT_F32:
+                fn = getattr(self._lib, f"cvs_{self._prefix}_run_batch_dev")
+                capi.check(fn(self._h, C.byref(b), mask, steer, theta, tm, arr, _stream_ptr(stream)))
+            else:
+                fn = getattr(self._lib, f"cvs_{self._prefix}_run_batch_dev_fmt")
+                capi.check(fn(self._h, C.byref(b), mask, steer, theta, tm, arr, _stream_ptr(stream), fmt))
         return {self._names[p]: outs[p] for p in planes}
 
     def run_pyramid(self, frames: torch.Tensor, levels: int, mask: int, **kw) -> List[Dict[str, torch.Tensor]]:
         """Every pyramid level stays resident on the device: level l+1 = pyr_down(level l), then one fused
-        launch per level (config 3 of BASELINE.json)."""
+        launch per level (config 3 of BASELINE.json).  Keyword arguments go to run(), out_dtype included; the levels
+        themselves (the next level's input) stay float32."""
         res, cur = [], _as_batch(frames)
         fuse = kw.pop("fuse_pyramid", True)
         for l in range(levels):
@@ -151,16 +180,21 @@ class G2Batch(_FusedBatch):
         super().__init__(width, spacing, device)
 
     def run_host(self, frames_host: torch.Tensor, mask: int, outs_host: Dict[int, torch.Tensor]):
-        """End-to-end host-buffer call (cvs_g2_run_batch_host): pinned host frames in, pinned host planes out."""
+        """End-to-end host-buffer call (cvs_g2_run_batch_host): pinned host frames in, pinned host planes out.  The
+        planes' dtype (float32, float16 or bfloat16, the same for all) selects the output format."""
         x = frames_host
         n, rows, cols = x.shape
+        fmt, es = _host_format(outs_host)
         arr = (C.c_void_p * capi.G2_NPLANES)()
         for p, t in outs_host.items():
             arr[p] = t.data_ptr()
         any_out = next(iter(outs_host.values()))
-        capi.check(self._lib.cvs_g2_run_batch_host(self._h, C.c_void_p(x.data_ptr()), n, rows, cols, x.stride(1) * 4,
-                                                   x.stride(0) * 4, mask, arr, any_out.stride(1) * 4,
-                                                   any_out.stride(0) * 4))
+        args = (self._h, C.c_void_p(x.data_ptr()), n, rows, cols, x.stride(1) * 4, x.stride(0) * 4, mask, arr,
+                any_out.stride(1) * es, any_out.stride(0) * es)
+        if fmt == capi.OUT_F32:
+            capi.check(self._lib.cvs_g2_run_batch_host(*args))
+        else:
+            capi.check(self._lib.cvs_g2_run_batch_host_fmt(*args, fmt))
 
 
 class G4Batch(_FusedBatch):
@@ -172,17 +206,22 @@ class G4Batch(_FusedBatch):
 
     def run_host(self, frames_host: torch.Tensor, mask: int, outs_host: Dict[int, torch.Tensor],
                  theta: Optional[float] = None):
-        """End-to-end host-buffer call (cvs_g4_run_batch_host).  theta=None steers at the G4 theta_d."""
+        """End-to-end host-buffer call (cvs_g4_run_batch_host).  theta=None steers at the G4 theta_d.  The planes' dtype
+        (float32, float16 or bfloat16, the same for all) selects the output format."""
         x = frames_host
         n, rows, cols = x.shape
+        fmt, es = _host_format(outs_host)
         arr = (C.c_void_p * capi.G4_NPLANES)()
         for p, t in outs_host.items():
             arr[p] = t.data_ptr()
         any_out = next(iter(outs_host.values()))
         src = capi.STEER_DOMINANT if theta is None else capi.STEER_SCALAR
-        capi.check(self._lib.cvs_g4_run_batch_host(self._h, C.c_void_p(x.data_ptr()), n, rows, cols, x.stride(1) * 4,
-                                                   x.stride(0) * 4, mask, src, float(theta or 0.0), arr,
-                                                   any_out.stride(1) * 4, any_out.stride(0) * 4))
+        args = (self._h, C.c_void_p(x.data_ptr()), n, rows, cols, x.stride(1) * 4, x.stride(0) * 4, mask, src,
+                float(theta or 0.0), arr, any_out.stride(1) * es, any_out.stride(0) * es)
+        if fmt == capi.OUT_F32:
+            capi.check(self._lib.cvs_g4_run_batch_host(*args))
+        else:
+            capi.check(self._lib.cvs_g4_run_batch_host_fmt(*args, fmt))
 
 
 def pyr_down(frames: torch.Tensor, band: Optional[Band] = None, out_rows: Optional[range] = None,

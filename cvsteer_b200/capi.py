@@ -37,6 +37,7 @@ G2_MASK_STEER5 = bit(G2T) | bit(H2T) | bit(E) | bit(MAG) | bit(PHASE)
 G4_MASK_BASIS = 0x000007FF
 G4_MASK_STEER = bit(G4T) | bit(H4T) | bit(MAG4) | bit(PHASE4)
 STEER_DOMINANT, STEER_SCALAR, STEER_MAP = 0, 1, 2
+OUT_F32, OUT_F16, OUT_BF16 = 0, 1, 2
 GATHER_NONE, GATHER_NCCL, GATHER_PEER_STORE, GATHER_PEER_COPY = 0, 1, 2, 3
 
 OK, ERR_INVALID_ARG, ERR_CUDA, ERR_NOT_SETUP, ERR_SIZE_MISMATCH, ERR_UNSUPPORTED = 0, -1, -2, -3, -4, -5
@@ -90,6 +91,10 @@ _SIGS = {
                                        C.POINTER(C.c_void_p), C.c_void_p]),
     "cvs_g4_run_batch_dev": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.c_uint, C.c_int, C.c_float, C.c_void_p,
                                        C.POINTER(C.c_void_p), C.c_void_p]),
+    "cvs_g2_run_batch_dev_fmt": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.c_uint, C.c_int, C.c_float, C.c_void_p,
+                                           C.POINTER(C.c_void_p), C.c_void_p, C.c_int]),
+    "cvs_g4_run_batch_dev_fmt": (C.c_int, [C.c_void_p, C.POINTER(Batch), C.c_uint, C.c_int, C.c_float, C.c_void_p,
+                                           C.POINTER(C.c_void_p), C.c_void_p, C.c_int]),
     "cvs_pyr_down_dev": (C.c_int, [C.c_int, C.POINTER(Batch), C.c_void_p, C.c_void_p]),
     "cvs_g2_run_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
                                         C.c_uint, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t]),
@@ -101,6 +106,11 @@ _SIGS = {
     "cvs_shared_free": (C.c_int, [C.c_int, C.c_void_p]),
     "cvs_g4_run_batch_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
                                         C.c_uint, C.c_int, C.c_float, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t]),
+    "cvs_g2_run_batch_host_fmt": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
+                                            C.c_uint, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t, C.c_int]),
+    "cvs_g4_run_batch_host_fmt": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
+                                            C.c_uint, C.c_int, C.c_float, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t,
+                                            C.c_int]),
     "cvs_to_u8_dev": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_float, C.c_void_p,
                                 C.c_size_t, C.c_size_t, C.c_void_p]),
     "cvs_g2_lines_u8_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_float,
@@ -108,6 +118,9 @@ _SIGS = {
     "cvs_g2_run_batch_host_multi": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_int,
                                               C.c_int, C.c_size_t, C.c_size_t, C.c_uint, C.POINTER(C.c_void_p), C.c_size_t,
                                               C.c_size_t]),
+    "cvs_g2_run_batch_host_multi_fmt": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.c_int, C.c_float, C.c_void_p, C.c_int,
+                                                  C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_uint, C.POINTER(C.c_void_p),
+                                                  C.c_size_t, C.c_size_t, C.c_int]),
     "cvs_g2_run_bands_host_multi": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_int,
                                               C.c_size_t, C.c_int, C.c_uint, C.POINTER(C.POINTER(C.c_void_p)),
                                               C.POINTER(C.c_size_t)]),

@@ -202,15 +202,18 @@ BatchGeom whole_frame_geom(const void* in, bool u8, int n, int rows, int cols, s
     return g;
 }
 
-int geom_from_batch(const cvs_batch* b, BatchGeom* g)
+// out_esz: bytes per output element (4 = fp32 planes, 2 = 16-bit planes)
+int geom_from_batch(const cvs_batch* b, BatchGeom* g, size_t out_esz = 4)
 {
     if (!b || !b->in) return fail(CVS_ERR_INVALID_ARG, "batch or batch->in is null");
     if (b->n <= 0 || b->rows <= 0 || b->cols <= 0) return fail(CVS_ERR_INVALID_ARG, "batch n/rows/cols must be positive");
     const size_t esz = b->in_is_u8 ? 1 : 4;
     if (b->in_pitch < (size_t)b->cols * esz) return fail(CVS_ERR_INVALID_ARG, "in_pitch %zu < cols*%zu", b->in_pitch, esz);
     if (b->out_pitch < (size_t)b->cols * 4 / 2) return fail(CVS_ERR_INVALID_ARG, "out_pitch too small");
-    if ((b->out_pitch & 3) || (b->out_frame_stride & 3) || (!b->in_is_u8 && ((b->in_pitch & 3) || (b->in_frame_stride & 3) || ((uintptr_t)b->in & 3))))
-        return fail(CVS_ERR_INVALID_ARG, "fp32 planes need 4-byte aligned base, pitch and frame stride");
+    if ((b->out_pitch & (out_esz - 1)) || (b->out_frame_stride & (out_esz - 1)) ||
+        (!b->in_is_u8 && ((b->in_pitch & 3) || (b->in_frame_stride & 3) || ((uintptr_t)b->in & 3))))
+        return fail(CVS_ERR_INVALID_ARG, out_esz == 4 ? "fp32 planes need 4-byte aligned base, pitch and frame stride"
+                                                      : "16-bit output planes need an even pitch and frame stride, fp32 input 4-byte alignment");
     *g = whole_frame_geom(b->in, b->in_is_u8 != 0, b->n, b->rows, b->cols, b->in_pitch, b->in_frame_stride, b->out_pitch,
                           b->out_frame_stride);
     if (b->next_level) {
@@ -273,6 +276,63 @@ int run_fused(Filter* f, const BatchGeom& g, unsigned mask, const SteerSpec& st,
         if (slot < 3) f->scratch_used[slot] = true, f->scratch_stream[slot] = stream;
     }
     CU_TRY(launch_basis_fused(f->family, f->taps, g, mask, st, outs, scratch, stream, &f->last));
+    return CVS_OK;
+}
+
+// run_fused with output planes in `fmt` (cvs_out_format; g.out_pitch / g.out_frame_stride in bytes of them).  The fused 16-bit
+// kernel when one exists for this launch; otherwise the fp32 kernel writes stream-ordered scratch in the angle map's layout
+// (4-byte elements, twice the outputs' pitch and frame stride, so CVS_STEER_MAP works unchanged), chunked by frames to bound
+// its size, and k_narrow rounds it into the caller's planes: the same bits either way.
+int run_fused_fmt(Filter* f, const BatchGeom& g, unsigned mask, const SteerSpec& st, void* const* outs, int fmt, cudaStream_t stream, int slot = 0,
+                  int nslots = 1)
+{
+    if (fmt == CVS_OUT_F32) return run_fused(f, g, mask, st, reinterpret_cast<float* const*>(outs), stream, slot, nslots);
+    CU_TRY(cudaSetDevice(f->device));
+    bool taken = false;
+    CU_TRY(launch_basis_fused16(f->family, fmt, f->taps, g, mask, st, outs, stream, &f->last, &taken));
+    if (taken) return CVS_OK;
+    const int nplanes = f->family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES;
+    int sel[MARCH_MAX_OUT_HOST], np = 0;
+    for (int p = 0; p < nplanes; ++p)
+        if (mask >> p & 1u) sel[np++] = p;
+    const int rows = g.out_row_end - g.out_row_begin;
+    if (np == 0 || rows <= 0) return fail(CVS_ERR_INVALID_ARG, "empty launch");
+    const size_t s_pitch = 2 * g.out_pitch, s_fs = g.n > 1 ? 2 * g.out_frame_stride : s_pitch * rows;
+    const size_t budget = 512ull << 20;  // scratch bytes per call (at least one frame)
+    int chunk = (int)std::min<size_t>((size_t)g.n, std::max<size_t>(1, budget / (s_fs * np)));
+    chunk = std::min(chunk, 65535 / np);  // k_narrow: frames x planes in gridDim.z
+    const size_t plane_bytes = (size_t)(chunk - 1) * s_fs + s_pitch * rows;
+    void* scratch = nullptr;
+    CU_TRY(cudaMallocAsync(&scratch, plane_bytes * np, stream));
+    int rc = CVS_OK;
+    for (int f0 = 0; f0 < g.n && rc == CVS_OK; f0 += chunk) {
+        const int nf = std::min(chunk, g.n - f0);
+        BatchGeom gc = g;
+        gc.n = nf;
+        gc.in = static_cast<const char*>(g.in) + (size_t)f0 * g.in_frame_stride;
+        gc.out_pitch = s_pitch, gc.out_frame_stride = s_fs;
+        if (g.next_level) gc.next_level = reinterpret_cast<float*>(reinterpret_cast<char*>(g.next_level) + (size_t)f0 * g.next_frame_stride);
+        SteerSpec sc = st;
+        if (sc.theta_map) sc.theta_map = reinterpret_cast<const float*>(reinterpret_cast<const char*>(st.theta_map) + (size_t)f0 * s_fs);
+        float* souts[MARCH_MAX_OUT_HOST] = {nullptr};
+        const float* src[MARCH_MAX_OUT_HOST];
+        void* dst[MARCH_MAX_OUT_HOST];
+        for (int i = 0; i < np; ++i) {
+            souts[sel[i]] = reinterpret_cast<float*>(static_cast<char*>(scratch) + (size_t)i * plane_bytes);
+            src[i] = souts[sel[i]];
+            dst[i] = static_cast<char*>(outs[sel[i]]) + (size_t)f0 * g.out_frame_stride;
+        }
+        rc = run_fused(f, gc, mask, sc, souts, stream, slot, nslots);
+        if (rc == CVS_OK) {
+            const cudaError_t e = launch_narrow(fmt, np, src, s_pitch, s_fs, dst, g.out_pitch, g.out_frame_stride, nf, rows, g.cols, stream);
+            if (e != cudaSuccess) rc = fail(CVS_ERR_CUDA, "narrow: %s", cudaGetErrorString(e));
+        }
+    }
+    const cudaError_t e = cudaFreeAsync(scratch, stream);
+    if (rc != CVS_OK) return rc;
+    CU_TRY(e);
+    const size_t len = strlen(f->last.name);
+    snprintf(f->last.name + len, sizeof(f->last.name) - len, "+narrow-%s", fmt == CVS_OUT_F16 ? "f16" : "bf16");
     return CVS_OK;
 }
 
@@ -586,12 +646,30 @@ extern "C" int cvs_g4_steer_map_host(cvs_g4* h, const float* theta, size_t theta
 }
 
 // ================================ device-resident batch path ================================
-static int run_batch_dev(Filter* f, const cvs_batch* b, unsigned mask, int steer_source, float theta, const float* theta_map,
-                         float* const* outs, void* stream)
+// 16-bit output layout (fmt != CVS_OUT_F32): checked before anything else, the handle included, and before any CUDA call
+// (nplanes: entries of `outs` that may be read)
+static int check_out16(int fmt, int cols, size_t out_pitch, unsigned mask, int nplanes, void* const* outs)
 {
+    if (fmt != CVS_OUT_F16 && fmt != CVS_OUT_BF16) return fail(CVS_ERR_INVALID_ARG, "out_format %d is not a cvs_out_format", fmt);
+    if (out_pitch < (size_t)cols * 2) return fail(CVS_ERR_INVALID_ARG, "out_pitch %zu < cols*2", out_pitch);
+    if (out_pitch & 1) return fail(CVS_ERR_INVALID_ARG, "16-bit planes need an even out_pitch (%zu)", out_pitch);
+    for (int p = 0; outs && p < nplanes; ++p)
+        if ((mask >> p & 1u) && ((uintptr_t)outs[p] & 1)) return fail(CVS_ERR_INVALID_ARG, "outs[%d] is not 2-byte aligned", p);
+    return CVS_OK;
+}
+
+static int run_batch_dev(Filter* f, const cvs_batch* b, unsigned mask, int steer_source, float theta, const float* theta_map,
+                         void* const* outs, void* stream, int fmt = CVS_OUT_F32)
+{
+    const size_t esz = fmt == CVS_OUT_F32 ? 4 : 2;
+    if (fmt != CVS_OUT_F32) {
+        if (!b) return fail(CVS_ERR_INVALID_ARG, "batch is null");
+        const int nplanes = f && f->family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES;  // no handle: the smaller family
+        if (int rc = check_out16(fmt, b->cols, b->out_pitch, mask, nplanes, outs)) return rc;
+    }
     if (!f) return fail(CVS_ERR_INVALID_ARG, "handle is null");
     BatchGeom g;
-    int rc = geom_from_batch(b, &g);
+    int rc = geom_from_batch(b, &g, esz);
     if (rc) return rc;
     rc = check_band(g, f->taps.width, g.full_rows);
     if (rc) return rc;
@@ -600,7 +678,7 @@ static int run_batch_dev(Filter* f, const cvs_batch* b, unsigned mask, int steer
     if (!outs) return fail(CVS_ERR_INVALID_ARG, "outs is null");
     for (int p = 0; p < nplanes; ++p)
         if ((mask >> p & 1u) && !outs[p]) return fail(CVS_ERR_INVALID_ARG, "outs[%d] is null but selected by mask", p);
-    if (b->out_pitch < (size_t)b->cols * 4) return fail(CVS_ERR_INVALID_ARG, "out_pitch %zu < cols*4", b->out_pitch);
+    if (b->out_pitch < (size_t)b->cols * esz) return fail(CVS_ERR_INVALID_ARG, "out_pitch %zu < cols*%zu", b->out_pitch, esz);
     if (steer_source < CVS_STEER_DOMINANT || steer_source > CVS_STEER_MAP) return fail(CVS_ERR_INVALID_ARG, "steer_source %d", steer_source);
     if (steer_source == CVS_STEER_MAP && !theta_map) return fail(CVS_ERR_INVALID_ARG, "theta_map is null");
     SteerSpec st{};
@@ -608,18 +686,28 @@ static int run_batch_dev(Filter* f, const cvs_batch* b, unsigned mask, int steer
     st.cos_t = std::cos(theta);
     st.sin_t = std::sin(theta);
     st.theta_map = theta_map;
-    return run_fused(f, g, mask, st, outs, static_cast<cudaStream_t>(stream));
+    return run_fused_fmt(f, g, mask, st, outs, fmt, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int cvs_g2_run_batch_dev(cvs_g2* h, const cvs_batch* b, unsigned mask, int steer_source, float theta_scalar,
                                     const float* theta_map, float* const* outs, void* stream)
 {
-    return run_batch_dev(reinterpret_cast<Filter*>(h), b, mask, steer_source, theta_scalar, theta_map, outs, stream);
+    return run_batch_dev(reinterpret_cast<Filter*>(h), b, mask, steer_source, theta_scalar, theta_map, reinterpret_cast<void* const*>(outs), stream);
 }
 extern "C" int cvs_g4_run_batch_dev(cvs_g4* h, const cvs_batch* b, unsigned mask, int steer_source, float theta_scalar,
                                     const float* theta_map, float* const* outs, void* stream)
 {
-    return run_batch_dev(reinterpret_cast<Filter*>(h), b, mask, steer_source, theta_scalar, theta_map, outs, stream);
+    return run_batch_dev(reinterpret_cast<Filter*>(h), b, mask, steer_source, theta_scalar, theta_map, reinterpret_cast<void* const*>(outs), stream);
+}
+extern "C" int cvs_g2_run_batch_dev_fmt(cvs_g2* h, const cvs_batch* b, unsigned mask, int steer_source, float theta_scalar,
+                                        const float* theta_map, void* const* outs, void* stream, int out_format)
+{
+    return run_batch_dev(reinterpret_cast<Filter*>(h), b, mask, steer_source, theta_scalar, theta_map, outs, stream, out_format);
+}
+extern "C" int cvs_g4_run_batch_dev_fmt(cvs_g4* h, const cvs_batch* b, unsigned mask, int steer_source, float theta_scalar,
+                                        const float* theta_map, void* const* outs, void* stream, int out_format)
+{
+    return run_batch_dev(reinterpret_cast<Filter*>(h), b, mask, steer_source, theta_scalar, theta_map, outs, stream, out_format);
 }
 
 extern "C" int cvs_pyr_down_dev(int device, const cvs_batch* b, float* out, void* stream)
@@ -643,15 +731,21 @@ extern "C" int cvs_pyr_down_dev(int device, const cvs_batch* b, float* out, void
 // Host-buffer batch: frames are processed in chunks on two streams so that the upload of chunk i+1, the kernel of
 // chunk i and the download of chunk i-1 overlap.
 namespace {
+// fmt: cvs_out_format of the host output planes (out_step / out_frame_stride in bytes of them)
 int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride, unsigned mask,
-                   int steer_source, float theta, float* const* outs, size_t out_step, size_t out_frame_stride)
+                   int steer_source, float theta, void* const* outs, size_t out_step, size_t out_frame_stride, int fmt = CVS_OUT_F32)
 {
+    const size_t esz = fmt == CVS_OUT_F32 ? 4 : 2;
+    if (fmt != CVS_OUT_F32) {
+        if (int rc = check_out16(fmt, cols, out_step, mask, family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES, outs)) return rc;
+        if (out_frame_stride & 1) return fail(CVS_ERR_INVALID_ARG, "16-bit planes need an even out_frame_stride (%zu)", out_frame_stride);
+    }
     if (!f || f->family != family || !in || !outs) return fail(CVS_ERR_INVALID_ARG, "null argument or wrong handle family");
     const int NPLANES = family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES;
     if (steer_source != CVS_STEER_DOMINANT && steer_source != CVS_STEER_SCALAR)
         return fail(CVS_ERR_INVALID_ARG, "host batches steer at theta_d or at one scalar angle (steer_source %d)", steer_source);
     if (n <= 0 || rows <= 0 || cols <= 0) return fail(CVS_ERR_INVALID_ARG, "n/rows/cols must be positive");
-    if (in_step < (size_t)cols * 4 || out_step < (size_t)cols * 4) return fail(CVS_ERR_INVALID_ARG, "step < cols*4");
+    if (in_step < (size_t)cols * 4 || out_step < (size_t)cols * esz) return fail(CVS_ERR_INVALID_ARG, "step < cols*%zu", esz);
     if (!mask || (mask >> NPLANES)) return fail(CVS_ERR_INVALID_ARG, "mask 0x%x", mask);
     int nout = 0;
     for (int p = 0; p < NPLANES; ++p)
@@ -661,13 +755,15 @@ int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int 
         }
     CU_TRY(cudaSetDevice(f->device));
     const size_t pitch = align_up((size_t)cols * 4, 128), fbytes = pitch * rows;
+    const size_t opitch = align_up((size_t)cols * esz, 128), obytes = opitch * rows;  // device output planes
     // chunk so that >= 4 chunks exist (pipeline depth) but each is large enough to amortise launch + copy latency
     int chunk = (int)((64ull << 20) / fbytes);
     if (chunk < 1) chunk = 1;
     if (chunk > (n + 3) / 4) chunk = (n + 3) / 4;
     if (chunk < 1) chunk = 1;
     const int NBUF = 3;
-    CU_TRY(f->work.reserve((size_t)NBUF * chunk * fbytes * (1 + nout)));
+    const size_t slot_bytes = (size_t)chunk * (fbytes + nout * obytes);
+    CU_TRY(f->work.reserve(NBUF * slot_bytes));
     cudaStream_t* streams = f->pipe;  // owned by the handle: they live on the handle's device
     for (int i = 0; i < NBUF; ++i)
         if (!streams[i]) CU_TRY(cudaStreamCreateWithFlags(&streams[i], cudaStreamNonBlocking));
@@ -680,7 +776,7 @@ int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int 
         const int nf = (n - f0 < chunk) ? (n - f0) : chunk;
         const int b = ci % NBUF;
         cudaStream_t s = streams[b];
-        char* base = static_cast<char*>(f->work.p) + (size_t)b * chunk * fbytes * (1 + nout);
+        char* base = static_cast<char*>(f->work.p) + (size_t)b * slot_bytes;
         float* din = reinterpret_cast<float*>(base);
         // 3-D copy: frames x rows x row-bytes
         cudaMemcpy3DParms cp{};
@@ -702,29 +798,30 @@ int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int 
                                          reinterpret_cast<const char*>(in) + (size_t)(f0 + k) * in_frame_stride, in_step, (size_t)cols * 4,
                                          rows, cudaMemcpyHostToDevice, s));
         }
-        float* douts[(int)CVS_G2_NPLANES > (int)CVS_G4_NPLANES ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES] = {nullptr};
+        void* douts[(int)CVS_G2_NPLANES > (int)CVS_G4_NPLANES ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES] = {nullptr};
         int slot = 0;
         for (int p = 0; p < NPLANES; ++p)
-            if (mask >> p & 1u) douts[p] = reinterpret_cast<float*>(base + (size_t)(1 + slot++) * chunk * fbytes);
-        BatchGeom g = whole_frame_geom(din, false, nf, rows, cols, pitch, fbytes, pitch, fbytes);
-        int rc = run_fused(f, g, mask, st, douts, s, b, NBUF);
+            if (mask >> p & 1u) douts[p] = base + (size_t)chunk * fbytes + (size_t)(slot++) * chunk * obytes;
+        BatchGeom g = whole_frame_geom(din, false, nf, rows, cols, pitch, fbytes, opitch, obytes);
+        int rc = run_fused_fmt(f, g, mask, st, douts, fmt, s, b, NBUF);
         if (rc) return rc;
+        const size_t row_bytes = (size_t)cols * esz;
         for (int p = 0; p < NPLANES; ++p)
             if (mask >> p & 1u) {
-                char* dst = reinterpret_cast<char*>(outs[p]) + (size_t)f0 * out_frame_stride;
-                if (pitch == (size_t)cols * 4 && out_step == pitch && out_frame_stride == fbytes) {
-                    CU_TRY(cudaMemcpyAsync(dst, douts[p], (size_t)nf * fbytes, cudaMemcpyDeviceToHost, s));
+                char* dst = static_cast<char*>(outs[p]) + (size_t)f0 * out_frame_stride;
+                if (opitch == row_bytes && out_step == opitch && out_frame_stride == obytes) {
+                    CU_TRY(cudaMemcpyAsync(dst, douts[p], (size_t)nf * obytes, cudaMemcpyDeviceToHost, s));
                 } else if (out_frame_stride % out_step == 0) {
                     cudaMemcpy3DParms cq{};
-                    cq.srcPtr = make_cudaPitchedPtr(douts[p], pitch, (size_t)cols * 4, rows);
-                    cq.dstPtr = make_cudaPitchedPtr(dst, out_step, (size_t)cols * 4, out_frame_stride / out_step);
-                    cq.extent = make_cudaExtent((size_t)cols * 4, rows, nf);
+                    cq.srcPtr = make_cudaPitchedPtr(douts[p], opitch, row_bytes, rows);
+                    cq.dstPtr = make_cudaPitchedPtr(dst, out_step, row_bytes, out_frame_stride / out_step);
+                    cq.extent = make_cudaExtent(row_bytes, rows, nf);
                     cq.kind = cudaMemcpyDeviceToHost;
                     CU_TRY(cudaMemcpy3DAsync(&cq, s));
                 } else {
                     for (int k = 0; k < nf; ++k)
-                        CU_TRY(cudaMemcpy2DAsync(dst + (size_t)k * out_frame_stride, out_step, reinterpret_cast<char*>(douts[p]) + (size_t)k * fbytes,
-                                                 pitch, (size_t)cols * 4, rows, cudaMemcpyDeviceToHost, s));
+                        CU_TRY(cudaMemcpy2DAsync(dst + (size_t)k * out_frame_stride, out_step, static_cast<char*>(douts[p]) + (size_t)k * obytes,
+                                                 opitch, row_bytes, rows, cudaMemcpyDeviceToHost, s));
                 }
             }
     }
@@ -736,15 +833,28 @@ int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int 
 extern "C" int cvs_g2_run_batch_host(cvs_g2* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
                                      unsigned mask, float* const* outs, size_t out_step, size_t out_frame_stride)
 {
-    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f, outs,
-                          out_step, out_frame_stride);
+    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f,
+                          reinterpret_cast<void* const*>(outs), out_step, out_frame_stride);
 }
 extern "C" int cvs_g4_run_batch_host(cvs_g4* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
                                      unsigned mask, int steer_source, float theta_scalar, float* const* outs, size_t out_step,
                                      size_t out_frame_stride)
 {
+    return run_batch_host(reinterpret_cast<Filter*>(h), 4, in, n, rows, cols, in_step, in_frame_stride, mask, steer_source, theta_scalar,
+                          reinterpret_cast<void* const*>(outs), out_step, out_frame_stride);
+}
+extern "C" int cvs_g2_run_batch_host_fmt(cvs_g2* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                         unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride, int out_format)
+{
+    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f, outs,
+                          out_step, out_frame_stride, out_format);
+}
+extern "C" int cvs_g4_run_batch_host_fmt(cvs_g4* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                         unsigned mask, int steer_source, float theta_scalar, void* const* outs, size_t out_step,
+                                         size_t out_frame_stride, int out_format)
+{
     return run_batch_host(reinterpret_cast<Filter*>(h), 4, in, n, rows, cols, in_step, in_frame_stride, mask, steer_source, theta_scalar, outs,
-                          out_step, out_frame_stride);
+                          out_step, out_frame_stride, out_format);
 }
 
 extern "C" int cvs_to_u8_dev(int device, const float* src, int n, int rows, int cols, size_t pitch, size_t frame_stride, float gain, uint8_t* dst,
@@ -847,10 +957,14 @@ extern "C" int cvs_g2_lines_u8_host(cvs_g2* h, const uint8_t* gray, int n, int r
     return CVS_OK;
 }
 
-extern "C" int cvs_g2_run_batch_host_multi(int n_devices, const int* devices, int width, float spacing, const float* in, int n, int rows,
-                                           int cols, size_t in_step, size_t in_frame_stride, unsigned mask, float* const* outs,
-                                           size_t out_step, size_t out_frame_stride)
+static int run_batch_host_multi(int n_devices, const int* devices, int width, float spacing, const float* in, int n, int rows, int cols,
+                                size_t in_step, size_t in_frame_stride, unsigned mask, void* const* outs, size_t out_step,
+                                size_t out_frame_stride, int fmt)
 {
+    if (fmt != CVS_OUT_F32) {
+        if (int rc = check_out16(fmt, cols, out_step, mask, CVS_G2_NPLANES, outs)) return rc;
+        if (out_frame_stride & 1) return fail(CVS_ERR_INVALID_ARG, "16-bit planes need an even out_frame_stride (%zu)", out_frame_stride);
+    }
     if (n_devices <= 0 || n_devices > 64 || !in || !outs || n <= 0) return fail(CVS_ERR_INVALID_ARG, "bad argument");
     const int per = (n + n_devices - 1) / n_devices;
     std::vector<std::thread> threads;
@@ -863,11 +977,10 @@ extern "C" int cvs_g2_run_batch_host_multi(int n_devices, const int* devices, in
             cvs_g2* h = nullptr;
             int r = cvs_g2_create(&h, devices ? devices[d] : d, width, spacing);
             if (r == CVS_OK) {
-                float* o[CVS_G2_NPLANES];
-                for (int p = 0; p < CVS_G2_NPLANES; ++p)
-                    o[p] = outs[p] ? reinterpret_cast<float*>(reinterpret_cast<char*>(outs[p]) + (size_t)f0 * out_frame_stride) : nullptr;
-                r = cvs_g2_run_batch_host(h, reinterpret_cast<const float*>(reinterpret_cast<const char*>(in) + (size_t)f0 * in_frame_stride), nf, rows,
-                                          cols, in_step, in_frame_stride, mask, o, out_step, out_frame_stride);
+                void* o[CVS_G2_NPLANES];
+                for (int p = 0; p < CVS_G2_NPLANES; ++p) o[p] = outs[p] ? static_cast<char*>(outs[p]) + (size_t)f0 * out_frame_stride : nullptr;
+                r = run_batch_host(reinterpret_cast<Filter*>(h), 2, reinterpret_cast<const float*>(reinterpret_cast<const char*>(in) + (size_t)f0 * in_frame_stride),
+                                   nf, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f, o, out_step, out_frame_stride, fmt);
             }
             if (r != CVS_OK) msg[d] = cvs_last_error();  // thread-local text: carry it back to the caller's thread
             rc[d] = r;
@@ -878,6 +991,21 @@ extern "C" int cvs_g2_run_batch_host_multi(int n_devices, const int* devices, in
     for (int d = 0; d < n_devices; ++d)
         if (rc[d] != CVS_OK) return fail(rc[d], "device %d: %s", devices ? devices[d] : d, msg[d].c_str());
     return CVS_OK;
+}
+
+extern "C" int cvs_g2_run_batch_host_multi(int n_devices, const int* devices, int width, float spacing, const float* in, int n, int rows,
+                                           int cols, size_t in_step, size_t in_frame_stride, unsigned mask, float* const* outs,
+                                           size_t out_step, size_t out_frame_stride)
+{
+    return run_batch_host_multi(n_devices, devices, width, spacing, in, n, rows, cols, in_step, in_frame_stride, mask,
+                                reinterpret_cast<void* const*>(outs), out_step, out_frame_stride, CVS_OUT_F32);
+}
+extern "C" int cvs_g2_run_batch_host_multi_fmt(int n_devices, const int* devices, int width, float spacing, const float* in, int n, int rows,
+                                               int cols, size_t in_step, size_t in_frame_stride, unsigned mask, void* const* outs,
+                                               size_t out_step, size_t out_frame_stride, int out_format)
+{
+    return run_batch_host_multi(n_devices, devices, width, spacing, in, n, rows, cols, in_step, in_frame_stride, mask, outs, out_step,
+                                out_frame_stride, out_format);
 }
 
 // ---- row bands of one very large image over several GPUs of this process -------------------------------------------

@@ -19,8 +19,11 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 
+#include <type_traits>
 #include <utility>
 
 #include "device_math.cuh"
@@ -193,10 +196,36 @@ __device__ __forceinline__ unsigned long long opaque64(unsigned long long v)
     return r;
 }
 
-template <unsigned MASK, int NPLANES>
+// 16-bit output planes (TOut = __half / __nv_bfloat16): the fp32 value the epilogue computed, rounded to nearest even at the
+// store -- bit for bit what torch.Tensor.to(float16 / bfloat16) makes of the fp32 plane (NaN stays NaN, fp16 overflow is +-inf)
+template <typename TOut>
+__device__ __forceinline__ unsigned short to_out16(float v)
+{
+    unsigned short h;
+    if constexpr (std::is_same_v<TOut, __half>) asm("cvt.rn.f16.f32 %0, %1;" : "=h"(h) : "f"(v));
+    else asm("cvt.rn.bf16.f32 %0, %1;" : "=h"(h) : "f"(v));
+    return h;
+}
+// two adjacent pixels packed by one instruction: v0 in the low half (lower address), v1 in the high half
+template <typename TOut>
+__device__ __forceinline__ unsigned to_out16x2(float v0, float v1)
+{
+    unsigned r;
+    if constexpr (std::is_same_v<TOut, __half>) asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(v1), "f"(v0));
+    else asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(v1), "f"(v0));
+    return r;
+}
+
+// The steering-angle map stays fp32 in the outputs' ELEMENT layout: with 16-bit outputs its byte offsets and row step are
+// twice the outputs' (kThetaScale), with fp32 outputs they are the same.
+template <typename TOut>
+inline constexpr long long kThetaScale = 4 / (long long)sizeof(TOut);
+
+template <unsigned MASK, int NPLANES, typename TOut = float>
 struct OutCursor {
+    static constexpr bool F32 = sizeof(TOut) == 4;
     unsigned long long base[NPLANES];
-    unsigned long long th_base;  // steering-angle map (same layout as the outputs); dead unless theta() is used
+    unsigned long long th_base;  // steering-angle map (same element layout as the outputs); dead unless theta() is used
     unsigned idx;                // element index of this thread's pixel relative to the bases
     unsigned pitch_elems;
     mutable float pend[NPLANES];  // two-pixel threads: the left pixel's value waits here for its neighbour (registers)
@@ -208,10 +237,10 @@ struct OutCursor {
         for (int q = 0; q < NPLANES; ++q)
             base[q] = (MASK >> q & 1u) ? opaque64((unsigned long long)(reinterpret_cast<char*>(a.out[q]) + band_off)) : 0ull;
         th_base = (MASK >> MARCH_SRC_SHIFT) == 2u /* CVS_STEER_MAP */
-                      ? opaque64((unsigned long long)(reinterpret_cast<const char*>(a.theta_map) + band_off))
+                      ? opaque64((unsigned long long)(reinterpret_cast<const char*>(a.theta_map) + kThetaScale<TOut> * band_off))
                       : 0ull;
         idx = (unsigned)x;
-        pitch_elems = (unsigned)(a.out_pitch >> 2);
+        pitch_elems = (unsigned)(a.out_pitch >> (F32 ? 2 : 1));
 #pragma unroll
         for (int k = 0; k < 3; ++k) mn[k] = __int_as_float(0x7f800000), mx[k] = __int_as_float(0xff800000);  // +inf / -inf
     }
@@ -219,14 +248,24 @@ struct OutCursor {
     // recompute that pixel and store the identical value to the identical address.
     __device__ __forceinline__ void put(const MarchArgs&, int q, float v) const
     {
-        asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %1, 4, %0;\n\tst.global.cs.f32 [a], %2;\n\t}" ::"l"(base[q]), "r"(idx), "f"(v) : "memory");
+        if constexpr (F32)
+            asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %1, 4, %0;\n\tst.global.cs.f32 [a], %2;\n\t}" ::"l"(base[q]), "r"(idx), "f"(v) : "memory");
+        else
+            asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %1, 2, %0;\n\tst.global.cs.b16 [a], %2;\n\t}" ::"l"(base[q]), "r"(idx), "h"(to_out16<TOut>(v))
+                         : "memory");
     }
-    // two adjacent pixels of one thread as one 8-byte store (x even, bases and pitch multiples of 8: host-checked)
+    // two adjacent pixels of one thread as one 8-byte (fp32) or 4-byte (16-bit) store (x even, bases and pitch multiples of the
+    // store width: host-checked)
     __device__ __forceinline__ void put2(const MarchArgs&, int q, float v0, float v1) const
     {
-        asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %1, 4, %0;\n\tst.global.cs.v2.f32 [a], {%2, %3};\n\t}" ::"l"(base[q]), "r"(idx), "f"(v0),
-                     "f"(v1)
-                     : "memory");
+        if constexpr (F32)
+            asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %1, 4, %0;\n\tst.global.cs.v2.f32 [a], {%2, %3};\n\t}" ::"l"(base[q]), "r"(idx), "f"(v0),
+                         "f"(v1)
+                         : "memory");
+        else
+            asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %1, 2, %0;\n\tst.global.cs.b32 [a], %2;\n\t}" ::"l"(base[q]), "r"(idx),
+                         "r"(to_out16x2<TOut>(v0, v1))
+                         : "memory");
     }
     // steering angle of this thread's pixel `rows_ahead` output rows below the current one
     __device__ __forceinline__ float theta(const MarchArgs&, int rows_ahead = 0) const
@@ -249,32 +288,36 @@ struct OutCursor {
     __device__ __forceinline__ void next_row() { idx += pitch_elems; }
 };
 
-template <int NPLANES>
-struct OutCursor<0u, NPLANES> {  // run-time mask: one shared byte offset, 64-bit add per plane at the store
+template <int NPLANES, typename TOut>
+struct OutCursor<0u, NPLANES, TOut> {  // run-time mask: one shared byte offset, 64-bit add per plane at the store
+    static constexpr bool F32 = sizeof(TOut) == 4;
     long long off, pitch;
     mutable float pend[NPLANES];
     mutable float mn[3], mx[3];
     __device__ __forceinline__ void track(int k, float v) const { mn[k] = fminf(mn[k], v), mx[k] = fmaxf(mx[k], v); }
-    __device__ __forceinline__ OutCursor(const MarchArgs& a, long long band_off, int x) : off(band_off + 4ll * x), pitch(a.out_pitch)
+    __device__ __forceinline__ OutCursor(const MarchArgs& a, long long band_off, int x)
+        : off(band_off + (long long)sizeof(TOut) * x), pitch(a.out_pitch)
     {
 #pragma unroll
         for (int k = 0; k < 3; ++k) mn[k] = __int_as_float(0x7f800000), mx[k] = __int_as_float(0xff800000);
     }
     __device__ __forceinline__ void put(const MarchArgs& a, int q, float v) const
     {
-        __stcs(reinterpret_cast<float*>(reinterpret_cast<char*>(a.out[q]) + off), v);
+        if constexpr (F32) __stcs(reinterpret_cast<float*>(reinterpret_cast<char*>(a.out[q]) + off), v);
+        else __stcs(reinterpret_cast<unsigned short*>(reinterpret_cast<char*>(a.out[q]) + off), to_out16<TOut>(v));
     }
     __device__ __forceinline__ void put2(const MarchArgs& a, int q, float v0, float v1) const
     {
-        __stcs(reinterpret_cast<float2*>(reinterpret_cast<char*>(a.out[q]) + off), make_float2(v0, v1));
+        if constexpr (F32) __stcs(reinterpret_cast<float2*>(reinterpret_cast<char*>(a.out[q]) + off), make_float2(v0, v1));
+        else __stcs(reinterpret_cast<unsigned*>(reinterpret_cast<char*>(a.out[q]) + off), to_out16x2<TOut>(v0, v1));
     }
     __device__ __forceinline__ float theta(const MarchArgs& a, int rows_ahead = 0) const
     {
-        return *reinterpret_cast<const float*>(reinterpret_cast<const char*>(a.theta_map) + off + rows_ahead * pitch);
+        return *reinterpret_cast<const float*>(reinterpret_cast<const char*>(a.theta_map) + kThetaScale<TOut> * (off + rows_ahead * pitch));
     }
     __device__ __forceinline__ float2 theta2(const MarchArgs& a, int rows_ahead = 0) const
     {
-        return *reinterpret_cast<const float2*>(reinterpret_cast<const char*>(a.theta_map) + off + rows_ahead * pitch);
+        return *reinterpret_cast<const float2*>(reinterpret_cast<const char*>(a.theta_map) + kThetaScale<TOut> * (off + rows_ahead * pitch));
     }
     __device__ __forceinline__ void next_row() { off += pitch; }
 };
@@ -423,7 +466,8 @@ __device__ __forceinline__ void emit_next_level(const float* tile, const MarchAr
 // PX = pixels (adjacent columns) per thread.  PX = 2 halves the per-pixel cost of everything that is per THREAD and row:
 // shared-memory loads (K + 1 values as 8-byte loads feed two pixels instead of K values feeding one), store instructions
 // and their 64-bit address arithmetic (one 8-byte store per plane for two pixels), loop control.
-template <class Fam, unsigned MASK /* 0 = use a.mask at run time */, bool USE_TMA, typename TIn, bool BAKED, int PX = 1>
+// TOut: element type of the output planes (float, or __half / __nv_bfloat16 rounded at the store; see OutCursor).
+template <class Fam, unsigned MASK /* 0 = use a.mask at run time */, bool USE_TMA, typename TIn, bool BAKED, int PX = 1, typename TOut = float>
 __global__ void __launch_bounds__(MARCH_TW / PX, (PX == 2 && CVS_PX2_MIN_CTAS > 0) ? CVS_PX2_MIN_CTAS : Fam::MIN_CTAS)
 k_march(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ MarchArgs a,
         const __grid_constant__ TapTable<Fam::NSETS, Fam::R> taps)
@@ -487,10 +531,12 @@ k_march(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ MarchA
         if (Fam::template reads_theta_map<MASK>(a)) {
             const int rows_here = min(BH, a.out_row_end - yb);
             const int seg = (min(TW, a.cols - x0) * 4) & ~15;
-            const char* tp = reinterpret_cast<const char*>(a.theta_map) + (long long)frame * a.out_frame_stride +
-                             (long long)(yb - a.out_row_origin) * a.out_pitch + 4ll * x0;
-            if (seg > 0 && ((reinterpret_cast<uintptr_t>(tp) | (uintptr_t)a.out_pitch) & 15) == 0)
-                for (int r = threadIdx.x; r < rows_here; r += NT) ptx::bulk_prefetch_l2(tp + (long long)r * a.out_pitch, (uint32_t)seg);
+            constexpr long long TS = kThetaScale<TOut>;  // map offsets in bytes of 4-byte elements
+            const long long th_pitch = TS * a.out_pitch;
+            const char* tp = reinterpret_cast<const char*>(a.theta_map) + TS * ((long long)frame * a.out_frame_stride) +
+                             TS * ((long long)(yb - a.out_row_origin) * a.out_pitch) + 4ll * x0;
+            if (seg > 0 && ((reinterpret_cast<uintptr_t>(tp) | (uintptr_t)th_pitch) & 15) == 0)
+                for (int r = threadIdx.x; r < rows_here; r += NT) ptx::bulk_prefetch_l2(tp + (long long)r * th_pitch, (uint32_t)seg);
         }
     }
 
@@ -600,7 +646,7 @@ k_march(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ MarchA
     const long long band_off = (long long)frame * a.out_frame_stride + (long long)(yb - a.out_row_origin) * a.out_pitch;
     // per-plane base registers only pay off while there are few planes (2 registers each); wide masks share one offset
     // (the same goes for the families whose nine 13-row windows leave no registers to spare: G4)
-    using Cursor = OutCursor<((__builtin_popcount(MASK & MARCH_PLANE_BITS) <= CVS_CURSOR_MAX_PLANES && !Fam::SHARED_ROW_PASS) ? MASK : 0u), Fam::NPLANES>;
+    using Cursor = OutCursor<((__builtin_popcount(MASK & MARCH_PLANE_BITS) <= CVS_CURSOR_MAX_PLANES && !Fam::SHARED_ROW_PASS) ? MASK : 0u), Fam::NPLANES, TOut>;
     Cursor cur(a, band_off, x);
     // point-wise epilogue of the row just finished by col_pass (+ the stores), then on to the next output row
     auto emit_row = [&](float th, float th_right = 0.f) {  // th_right: the right pixel's steering angle (two-pixel @map kernels)

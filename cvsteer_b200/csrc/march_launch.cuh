@@ -78,12 +78,12 @@ static void fill_tap_table(const FamilyTaps& ft, TapTable<Fam::NSETS, Fam::R>& t
     for (int i = 0; i <= Fam::R; ++i) tt.t[Fam::kScaledSet][i] = scaled[Fam::R + i];
 }
 
-template <class Fam, unsigned MASK, bool TMA, typename TIn, bool BAKED, int PX = 1>
+template <class Fam, unsigned MASK, bool TMA, typename TIn, bool BAKED, int PX = 1, typename TOut = float>
 static cudaError_t launch_march_one(const CUtensorMap& tm, const MarchArgs& a, const TapTable<Fam::NSETS, Fam::R>& tt, dim3 grid,
                                     cudaStream_t stream, LaunchInfo* info, const char* name)
 {
     constexpr int smem = march_smem_bytes(Fam::R, Fam::BH, TMA && sizeof(TIn) == 1);
-    auto kfn = k_march<Fam, MASK, TMA, TIn, BAKED, PX>;
+    auto kfn = k_march<Fam, MASK, TMA, TIn, BAKED, PX, TOut>;
     // Function attributes are per DEVICE (context): one flag per (instantiation, device).  The 8-bit TMA variants ask for
     // more than the 48 KB default, so a process that drives several GPUs must set them on each one.
     static std::atomic<unsigned long long> done[4];  // 256 devices

@@ -222,6 +222,28 @@ CVS_API int cvs_g2_run_batch_dev(cvs_g2* h, const cvs_batch* b, unsigned mask, i
 CVS_API int cvs_g4_run_batch_dev(cvs_g4* h, const cvs_batch* b, unsigned mask, int steer_source,
                                  float theta_scalar, const float* theta_map, float* const* outs, void* stream);
 
+/* ---- 16-bit output planes ----
+ * The *_fmt entry points below take the same arguments as their fp32 counterparts plus `out_format`; one format applies to
+ * every output plane of a call.  Contract: a 16-bit plane is, bit for bit, the fp32 plane the same call writes with
+ * CVS_OUT_F32, rounded to nearest even into the chosen format (what torch.Tensor.to(torch.float16 / torch.bfloat16) does
+ * to that fp32 plane): NaN stays NaN, and fp16 overflow gives +-inf as IEEE specifies.
+ *   - CVS_OUT_F16: 11 significant bits, finite up to 65504.  The quadratic planes (c1..c3, strength, E) of 8-bit-range
+ *     images reach 1e5 and overflow; scale such inputs so those planes stay below 65504, e.g. to [0,1].
+ *   - CVS_OUT_BF16: any fp32 range at 8 significant bits (about 3 significant digits; half an ulp of an angle near pi is
+ *     8e-3 rad, against 9.8e-4 rad in fp16).
+ * Layout: out_pitch / out_frame_stride are bytes of the 16-bit planes (out_pitch >= cols*2; out_pitch and every plane
+ * 2-byte aligned).  The CVS_STEER_MAP angle map stays fp32 in the outputs' ELEMENT layout, so its byte pitch and frame
+ * stride are twice the outputs'.  `next_level` stays fp32 and is unchanged (it is the next level's input).
+ * Speed: every mask/source pair with a fused kernel above has a fused 16-bit twin (it stores 2 bytes per pixel and plane;
+ * two-pixel kernels need 4-byte aligned planes / out_pitch / out_frame_stride).  Everything else -- the cooperative loader,
+ * 8-bit input, other taps, other masks, a layout misaligned for the store width -- runs the fp32 kernel into stream-ordered
+ * scratch on the call's stream and narrows it, with the same bits.  CVS_OUT_F32 is exactly the fp32 call. */
+typedef enum cvs_out_format { CVS_OUT_F32 = 0, CVS_OUT_F16 = 1, CVS_OUT_BF16 = 2 } cvs_out_format;
+CVS_API int cvs_g2_run_batch_dev_fmt(cvs_g2* h, const cvs_batch* b, unsigned mask, int steer_source, float theta_scalar,
+                                     const float* theta_map, void* const* outs, void* stream, int out_format);
+CVS_API int cvs_g4_run_batch_dev_fmt(cvs_g4* h, const cvs_batch* b, unsigned mask, int steer_source, float theta_scalar,
+                                     const float* theta_map, void* const* outs, void* stream, int out_format);
+
 /* Pyramid level l -> l+1 on the device.  No reference counterpart; defined as cv::pyrDown:
  * [1 4 6 4 1]^2/256, BORDER_REFLECT_101, even samples, out size ((cols+1)/2, (rows+1)/2).
  * Band fields of `b` apply to the INPUT level; outputs rows [out_row_begin,out_row_end) are in the
@@ -242,6 +264,15 @@ CVS_API int cvs_g4_run_batch_host(cvs_g4* h, const float* in, int n, int rows, i
                                   size_t in_frame_stride, unsigned mask, int steer_source, float theta_scalar,
                                   float* const* outs, size_t out_step, size_t out_frame_stride);
 
+/* 16-bit host-buffer batches (see cvs_out_format): outs are host planes of the chosen format, out_step / out_frame_stride
+ * in bytes of them; downloads move 2 bytes per pixel and plane, dense rows (out_step == cols*2 == a multiple of 128) still
+ * as one linear copy per plane and chunk. */
+CVS_API int cvs_g2_run_batch_host_fmt(cvs_g2* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                      unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride, int out_format);
+CVS_API int cvs_g4_run_batch_host_fmt(cvs_g4* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                      unsigned mask, int steer_source, float theta_scalar, void* const* outs, size_t out_step,
+                                      size_t out_frame_stride, int out_format);
+
 /* ---- the callers' 8-bit post-processing (reference example/steer.cpp:92-104, test/test.cpp:93-95), on the device ----
  * gain > 0: Mat::convertTo(CV_8UC1, gain); gain <= 0: cv::normalize(src, dst, 0, 255, NORM_MINMAX, CV_8UC1), per frame. */
 CVS_API int cvs_to_u8_dev(int device, const float* src, int n, int rows, int cols, size_t pitch, size_t frame_stride, float gain,
@@ -261,6 +292,11 @@ CVS_API int cvs_g2_lines_u8_host(cvs_g2* h, const uint8_t* gray, int n, int rows
 CVS_API int cvs_g2_run_batch_host_multi(int n_devices, const int* devices, int width, float spacing, const float* in, int n,
                                         int rows, int cols, size_t in_step, size_t in_frame_stride, unsigned mask,
                                         float* const* outs, size_t out_step, size_t out_frame_stride);
+
+/* 16-bit twin of cvs_g2_run_batch_host_multi (see cvs_out_format) */
+CVS_API int cvs_g2_run_batch_host_multi_fmt(int n_devices, const int* devices, int width, float spacing, const float* in, int n,
+                                            int rows, int cols, size_t in_step, size_t in_frame_stride, unsigned mask,
+                                            void* const* outs, size_t out_step, size_t out_frame_stride, int out_format);
 
 /* The row-band plan both band paths use (this library's multi-GPU entry point below and cvsteer_b200/multi.py), for
  * callers that shard one huge image over one process per GPU themselves.  Band edges sit on multiples of 2^(levels-1)
