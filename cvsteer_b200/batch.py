@@ -70,6 +70,17 @@ def _host_format(outs_host: Dict[int, torch.Tensor]):
     return _out_format(dt), torch.empty((), dtype=dt).element_size()
 
 
+def _host_frames(x: torch.Tensor):
+    """(8-bit?, row step, frame step in bytes) of the host frames of one run_host call: float32 or uint8, rows of unit stride.
+    Checked here because the C calls take raw pointers and steps: any other layout would be read as the wrong bytes."""
+    if x.is_cuda or x.dtype not in (torch.float32, torch.uint8):
+        raise capi.CvsError(capi.ERR_INVALID_ARG, f"host frames are a CPU tensor of float32 or uint8, not {x.dtype} on {x.device}")
+    if x.stride(-1) != 1:
+        raise capi.CvsError(capi.ERR_INVALID_ARG, f"host frames need rows of unit stride, got strides {tuple(x.stride())}")
+    es = x.element_size()
+    return x.dtype == torch.uint8, x.stride(1) * es, x.stride(0) * es
+
+
 def _stream_ptr(stream):
     s = stream if stream is not None else torch.cuda.current_stream()
     return C.c_void_p(s.cuda_stream)
@@ -181,17 +192,21 @@ class G2Batch(_FusedBatch):
 
     def run_host(self, frames_host: torch.Tensor, mask: int, outs_host: Dict[int, torch.Tensor]):
         """End-to-end host-buffer call (cvs_g2_run_batch_host): pinned host frames in, pinned host planes out.  The
-        planes' dtype (float32, float16 or bfloat16, the same for all) selects the output format."""
+        planes' dtype (float32, float16 or bfloat16, the same for all) selects the output format.  uint8 frames go up as
+        bytes (cvs_g2_run_batch_host_u8) and give the planes of the same frames as float32."""
         x = frames_host
         n, rows, cols = x.shape
+        u8, step, fstride = _host_frames(x)
         fmt, es = _host_format(outs_host)
         arr = (C.c_void_p * capi.G2_NPLANES)()
         for p, t in outs_host.items():
             arr[p] = t.data_ptr()
         any_out = next(iter(outs_host.values()))
-        args = (self._h, C.c_void_p(x.data_ptr()), n, rows, cols, x.stride(1) * 4, x.stride(0) * 4, mask, arr,
+        args = (self._h, C.c_void_p(x.data_ptr()), n, rows, cols, step, fstride, mask, arr,
                 any_out.stride(1) * es, any_out.stride(0) * es)
-        if fmt == capi.OUT_F32:
+        if u8:
+            capi.check(self._lib.cvs_g2_run_batch_host_u8(*args, fmt))
+        elif fmt == capi.OUT_F32:
             capi.check(self._lib.cvs_g2_run_batch_host(*args))
         else:
             capi.check(self._lib.cvs_g2_run_batch_host_fmt(*args, fmt))
@@ -207,18 +222,21 @@ class G4Batch(_FusedBatch):
     def run_host(self, frames_host: torch.Tensor, mask: int, outs_host: Dict[int, torch.Tensor],
                  theta: Optional[float] = None):
         """End-to-end host-buffer call (cvs_g4_run_batch_host).  theta=None steers at the G4 theta_d.  The planes' dtype
-        (float32, float16 or bfloat16, the same for all) selects the output format."""
+        (float32, float16 or bfloat16, the same for all) selects the output format; uint8 frames as in G2Batch.run_host."""
         x = frames_host
         n, rows, cols = x.shape
+        u8, step, fstride = _host_frames(x)
         fmt, es = _host_format(outs_host)
         arr = (C.c_void_p * capi.G4_NPLANES)()
         for p, t in outs_host.items():
             arr[p] = t.data_ptr()
         any_out = next(iter(outs_host.values()))
         src = capi.STEER_DOMINANT if theta is None else capi.STEER_SCALAR
-        args = (self._h, C.c_void_p(x.data_ptr()), n, rows, cols, x.stride(1) * 4, x.stride(0) * 4, mask, src,
+        args = (self._h, C.c_void_p(x.data_ptr()), n, rows, cols, step, fstride, mask, src,
                 float(theta or 0.0), arr, any_out.stride(1) * es, any_out.stride(0) * es)
-        if fmt == capi.OUT_F32:
+        if u8:
+            capi.check(self._lib.cvs_g4_run_batch_host_u8(*args, fmt))
+        elif fmt == capi.OUT_F32:
             capi.check(self._lib.cvs_g4_run_batch_host(*args))
         else:
             capi.check(self._lib.cvs_g4_run_batch_host_fmt(*args, fmt))

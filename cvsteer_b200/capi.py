@@ -111,6 +111,11 @@ _SIGS = {
     "cvs_g4_run_batch_host_fmt": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
                                             C.c_uint, C.c_int, C.c_float, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t,
                                             C.c_int]),
+    "cvs_g2_run_batch_host_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
+                                           C.c_uint, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t, C.c_int]),
+    "cvs_g4_run_batch_host_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t,
+                                           C.c_uint, C.c_int, C.c_float, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t,
+                                           C.c_int]),
     "cvs_to_u8_dev": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_float, C.c_void_p,
                                 C.c_size_t, C.c_size_t, C.c_void_p]),
     "cvs_g2_lines_u8_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_float,
@@ -121,6 +126,9 @@ _SIGS = {
     "cvs_g2_run_batch_host_multi_fmt": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.c_int, C.c_float, C.c_void_p, C.c_int,
                                                   C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_uint, C.POINTER(C.c_void_p),
                                                   C.c_size_t, C.c_size_t, C.c_int]),
+    "cvs_g2_run_batch_host_multi_u8": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.c_int, C.c_float, C.c_void_p, C.c_int,
+                                                 C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_uint, C.POINTER(C.c_void_p),
+                                                 C.c_size_t, C.c_size_t, C.c_int]),
     "cvs_g2_run_bands_host_multi": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_int,
                                               C.c_size_t, C.c_int, C.c_uint, C.POINTER(C.POINTER(C.c_void_p)),
                                               C.POINTER(C.c_size_t)]),

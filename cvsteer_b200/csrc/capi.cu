@@ -731,11 +731,23 @@ extern "C" int cvs_pyr_down_dev(int device, const cvs_batch* b, float* out, void
 // Host-buffer batch: frames are processed in chunks on two streams so that the upload of chunk i+1, the kernel of
 // chunk i and the download of chunk i-1 overlap.
 namespace {
-// fmt: cvs_out_format of the host output planes (out_step / out_frame_stride in bytes of them)
-int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride, unsigned mask,
-                   int steer_source, float theta, void* const* outs, size_t out_step, size_t out_frame_stride, int fmt = CVS_OUT_F32)
+// The input layout of the 8-bit entry points, checked before anything else (the handle included) and before any CUDA call, as
+// the 16-bit output layout is (check_out16)
+int check_in_u8(const void* in, int cols, size_t in_step)
 {
-    const size_t esz = fmt == CVS_OUT_F32 ? 4 : 2;
+    if (!in) return fail(CVS_ERR_INVALID_ARG, "in is null");
+    if (in_step < (size_t)cols) return fail(CVS_ERR_INVALID_ARG, "in_step %zu < cols", in_step);
+    return CVS_OK;
+}
+
+// in_u8: 8-bit frames (in_step / in_frame_stride in bytes of them), else fp32; the device holds them in the same element type.
+// fmt: cvs_out_format of the host output planes (out_step / out_frame_stride in bytes of them)
+int run_batch_host(Filter* f, int family, const void* in, bool in_u8, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                   unsigned mask, int steer_source, float theta, void* const* outs, size_t out_step, size_t out_frame_stride, int fmt = CVS_OUT_F32)
+{
+    const size_t esz = fmt == CVS_OUT_F32 ? 4 : 2, in_esz = in_u8 ? 1 : 4;
+    if (in_u8)
+        if (int rc = check_in_u8(in, cols, in_step)) return rc;
     if (fmt != CVS_OUT_F32) {
         if (int rc = check_out16(fmt, cols, out_step, mask, family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES, outs)) return rc;
         if (out_frame_stride & 1) return fail(CVS_ERR_INVALID_ARG, "16-bit planes need an even out_frame_stride (%zu)", out_frame_stride);
@@ -745,7 +757,8 @@ int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int 
     if (steer_source != CVS_STEER_DOMINANT && steer_source != CVS_STEER_SCALAR)
         return fail(CVS_ERR_INVALID_ARG, "host batches steer at theta_d or at one scalar angle (steer_source %d)", steer_source);
     if (n <= 0 || rows <= 0 || cols <= 0) return fail(CVS_ERR_INVALID_ARG, "n/rows/cols must be positive");
-    if (in_step < (size_t)cols * 4 || out_step < (size_t)cols * esz) return fail(CVS_ERR_INVALID_ARG, "step < cols*%zu", esz);
+    if (in_step < (size_t)cols * in_esz) return fail(CVS_ERR_INVALID_ARG, "in_step < cols*%zu", in_esz);
+    if (out_step < (size_t)cols * esz) return fail(CVS_ERR_INVALID_ARG, "step < cols*%zu", esz);
     if (!mask || (mask >> NPLANES)) return fail(CVS_ERR_INVALID_ARG, "mask 0x%x", mask);
     int nout = 0;
     for (int p = 0; p < NPLANES; ++p)
@@ -754,15 +767,24 @@ int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int 
             ++nout;
         }
     CU_TRY(cudaSetDevice(f->device));
-    const size_t pitch = align_up((size_t)cols * 4, 128), fbytes = pitch * rows;
+    const size_t in_row = (size_t)cols * in_esz, pitch = align_up(in_row, 128), fbytes = pitch * rows;  // device input frames
     const size_t opitch = align_up((size_t)cols * esz, 128), obytes = opitch * rows;  // device output planes
-    // chunk so that >= 4 chunks exist (pipeline depth) but each is large enough to amortise launch + copy latency
-    int chunk = (int)((64ull << 20) / fbytes);
+    // G4 steering at a scalar angle into fp32 planes: with the default taps the fp32-frame launch folds the steering factors
+    // into the baked column taps (G4Fam::prescaled), which the fp32-output 8-bit kernel does not, so the two differ in the
+    // last bits.  There the 8-bit chunk is widened on the device and runs the fp32-frame launch, which keeps the contract
+    // (the planes of the widened frames).  Every 16-bit format has fused 8-bit kernels with the same taps as the fp32 ones.
+    const bool widen = in_u8 && fmt == CVS_OUT_F32 && family == 4 && steer_source == CVS_STEER_SCALAR;
+    const size_t wpitch = align_up((size_t)cols * 4, 128), wbytes = widen ? wpitch * rows : 0;  // fp32 frames; widened ones
+    // chunk so that >= 4 chunks exist (pipeline depth) but each is large enough to amortise launch + copy latency: 64 MB of
+    // fp32 frames.  8-bit frames count as the fp32 frames they stand for, so 1-byte input does not make chunks four times
+    // larger and the pipeline shorter (sizing by input + output bytes instead made the chunks of narrow outputs larger as well,
+    // measured 3-7 % slower end to end; DESIGN.md section 11)
+    int chunk = (int)((64ull << 20) / (wpitch * rows));
     if (chunk < 1) chunk = 1;
     if (chunk > (n + 3) / 4) chunk = (n + 3) / 4;
     if (chunk < 1) chunk = 1;
     const int NBUF = 3;
-    const size_t slot_bytes = (size_t)chunk * (fbytes + nout * obytes);
+    const size_t slot_bytes = (size_t)chunk * (fbytes + wbytes + nout * obytes);
     CU_TRY(f->work.reserve(NBUF * slot_bytes));
     cudaStream_t* streams = f->pipe;  // owned by the handle: they live on the handle's device
     for (int i = 0; i < NBUF; ++i)
@@ -777,32 +799,36 @@ int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int 
         const int b = ci % NBUF;
         cudaStream_t s = streams[b];
         char* base = static_cast<char*>(f->work.p) + (size_t)b * slot_bytes;
-        float* din = reinterpret_cast<float*>(base);
+        char* din = base;
         // 3-D copy: frames x rows x row-bytes
         cudaMemcpy3DParms cp{};
-        cp.srcPtr = make_cudaPitchedPtr(const_cast<char*>(reinterpret_cast<const char*>(in)) + (size_t)f0 * in_frame_stride, in_step,
-                                        (size_t)cols * 4, in_frame_stride / in_step);
-        cp.dstPtr = make_cudaPitchedPtr(din, pitch, (size_t)cols * 4, rows);
-        cp.extent = make_cudaExtent((size_t)cols * 4, rows, nf);
+        cp.srcPtr = make_cudaPitchedPtr(const_cast<char*>(static_cast<const char*>(in)) + (size_t)f0 * in_frame_stride, in_step, in_row,
+                                        in_frame_stride / in_step);
+        cp.dstPtr = make_cudaPitchedPtr(din, pitch, in_row, rows);
+        cp.extent = make_cudaExtent(in_row, rows, nf);
         cp.kind = cudaMemcpyHostToDevice;
         // fully contiguous on both sides (the common case: dense frames whose row is a multiple of 128 bytes): one linear copy,
         // which the copy engine streams a little faster than the equivalent pitched 3-D copy
-        const bool in_dense = pitch == (size_t)cols * 4 && in_step == pitch && in_frame_stride == fbytes;
+        const bool in_dense = pitch == in_row && in_step == pitch && in_frame_stride == fbytes;
         if (in_dense) {
-            CU_TRY(cudaMemcpyAsync(din, reinterpret_cast<const char*>(in) + (size_t)f0 * in_frame_stride, (size_t)nf * fbytes, cudaMemcpyHostToDevice, s));
+            CU_TRY(cudaMemcpyAsync(din, static_cast<const char*>(in) + (size_t)f0 * in_frame_stride, (size_t)nf * fbytes, cudaMemcpyHostToDevice, s));
         } else if (in_frame_stride % in_step == 0) {
             CU_TRY(cudaMemcpy3DAsync(&cp, s));
         } else {
             for (int k = 0; k < nf; ++k)
-                CU_TRY(cudaMemcpy2DAsync(reinterpret_cast<char*>(din) + (size_t)k * fbytes, pitch,
-                                         reinterpret_cast<const char*>(in) + (size_t)(f0 + k) * in_frame_stride, in_step, (size_t)cols * 4,
-                                         rows, cudaMemcpyHostToDevice, s));
+                CU_TRY(cudaMemcpy2DAsync(din + (size_t)k * fbytes, pitch, static_cast<const char*>(in) + (size_t)(f0 + k) * in_frame_stride, in_step,
+                                         in_row, rows, cudaMemcpyHostToDevice, s));
         }
         void* douts[(int)CVS_G2_NPLANES > (int)CVS_G4_NPLANES ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES] = {nullptr};
         int slot = 0;
         for (int p = 0; p < NPLANES; ++p)
             if (mask >> p & 1u) douts[p] = base + (size_t)chunk * fbytes + (size_t)(slot++) * chunk * obytes;
-        BatchGeom g = whole_frame_geom(din, false, nf, rows, cols, pitch, fbytes, opitch, obytes);
+        BatchGeom g = whole_frame_geom(din, in_u8, nf, rows, cols, pitch, fbytes, opitch, obytes);
+        if (widen) {
+            float* dw = reinterpret_cast<float*>(base + (size_t)chunk * (fbytes + nout * obytes));
+            CU_TRY(launch_widen(reinterpret_cast<const unsigned char*>(din), pitch, fbytes, dw, wpitch, wbytes, nf, rows, cols, s));
+            g = whole_frame_geom(dw, false, nf, rows, cols, wpitch, wbytes, opitch, obytes);
+        }
         int rc = run_fused_fmt(f, g, mask, st, douts, fmt, s, b, NBUF);
         if (rc) return rc;
         const size_t row_bytes = (size_t)cols * esz;
@@ -833,27 +859,40 @@ int run_batch_host(Filter* f, int family, const float* in, int n, int rows, int 
 extern "C" int cvs_g2_run_batch_host(cvs_g2* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
                                      unsigned mask, float* const* outs, size_t out_step, size_t out_frame_stride)
 {
-    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f,
+    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, false, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f,
                           reinterpret_cast<void* const*>(outs), out_step, out_frame_stride);
 }
 extern "C" int cvs_g4_run_batch_host(cvs_g4* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
                                      unsigned mask, int steer_source, float theta_scalar, float* const* outs, size_t out_step,
                                      size_t out_frame_stride)
 {
-    return run_batch_host(reinterpret_cast<Filter*>(h), 4, in, n, rows, cols, in_step, in_frame_stride, mask, steer_source, theta_scalar,
+    return run_batch_host(reinterpret_cast<Filter*>(h), 4, in, false, n, rows, cols, in_step, in_frame_stride, mask, steer_source, theta_scalar,
                           reinterpret_cast<void* const*>(outs), out_step, out_frame_stride);
 }
 extern "C" int cvs_g2_run_batch_host_fmt(cvs_g2* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
                                          unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride, int out_format)
 {
-    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f, outs,
+    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, false, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f, outs,
                           out_step, out_frame_stride, out_format);
 }
 extern "C" int cvs_g4_run_batch_host_fmt(cvs_g4* h, const float* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
                                          unsigned mask, int steer_source, float theta_scalar, void* const* outs, size_t out_step,
                                          size_t out_frame_stride, int out_format)
 {
-    return run_batch_host(reinterpret_cast<Filter*>(h), 4, in, n, rows, cols, in_step, in_frame_stride, mask, steer_source, theta_scalar, outs,
+    return run_batch_host(reinterpret_cast<Filter*>(h), 4, in, false, n, rows, cols, in_step, in_frame_stride, mask, steer_source, theta_scalar, outs,
+                          out_step, out_frame_stride, out_format);
+}
+extern "C" int cvs_g2_run_batch_host_u8(cvs_g2* h, const uint8_t* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                        unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride, int out_format)
+{
+    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, true, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f, outs,
+                          out_step, out_frame_stride, out_format);
+}
+extern "C" int cvs_g4_run_batch_host_u8(cvs_g4* h, const uint8_t* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                        unsigned mask, int steer_source, float theta_scalar, void* const* outs, size_t out_step,
+                                        size_t out_frame_stride, int out_format)
+{
+    return run_batch_host(reinterpret_cast<Filter*>(h), 4, in, true, n, rows, cols, in_step, in_frame_stride, mask, steer_source, theta_scalar, outs,
                           out_step, out_frame_stride, out_format);
 }
 
@@ -957,10 +996,12 @@ extern "C" int cvs_g2_lines_u8_host(cvs_g2* h, const uint8_t* gray, int n, int r
     return CVS_OK;
 }
 
-static int run_batch_host_multi(int n_devices, const int* devices, int width, float spacing, const float* in, int n, int rows, int cols,
-                                size_t in_step, size_t in_frame_stride, unsigned mask, void* const* outs, size_t out_step,
+static int run_batch_host_multi(int n_devices, const int* devices, int width, float spacing, const void* in, bool in_u8, int n, int rows,
+                                int cols, size_t in_step, size_t in_frame_stride, unsigned mask, void* const* outs, size_t out_step,
                                 size_t out_frame_stride, int fmt)
 {
+    if (in_u8)
+        if (int rc = check_in_u8(in, cols, in_step)) return rc;
     if (fmt != CVS_OUT_F32) {
         if (int rc = check_out16(fmt, cols, out_step, mask, CVS_G2_NPLANES, outs)) return rc;
         if (out_frame_stride & 1) return fail(CVS_ERR_INVALID_ARG, "16-bit planes need an even out_frame_stride (%zu)", out_frame_stride);
@@ -979,8 +1020,8 @@ static int run_batch_host_multi(int n_devices, const int* devices, int width, fl
             if (r == CVS_OK) {
                 void* o[CVS_G2_NPLANES];
                 for (int p = 0; p < CVS_G2_NPLANES; ++p) o[p] = outs[p] ? static_cast<char*>(outs[p]) + (size_t)f0 * out_frame_stride : nullptr;
-                r = run_batch_host(reinterpret_cast<Filter*>(h), 2, reinterpret_cast<const float*>(reinterpret_cast<const char*>(in) + (size_t)f0 * in_frame_stride),
-                                   nf, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f, o, out_step, out_frame_stride, fmt);
+                r = run_batch_host(reinterpret_cast<Filter*>(h), 2, static_cast<const char*>(in) + (size_t)f0 * in_frame_stride, in_u8, nf, rows, cols,
+                                   in_step, in_frame_stride, mask, CVS_STEER_DOMINANT, 0.f, o, out_step, out_frame_stride, fmt);
             }
             if (r != CVS_OK) msg[d] = cvs_last_error();  // thread-local text: carry it back to the caller's thread
             rc[d] = r;
@@ -997,14 +1038,21 @@ extern "C" int cvs_g2_run_batch_host_multi(int n_devices, const int* devices, in
                                            int cols, size_t in_step, size_t in_frame_stride, unsigned mask, float* const* outs,
                                            size_t out_step, size_t out_frame_stride)
 {
-    return run_batch_host_multi(n_devices, devices, width, spacing, in, n, rows, cols, in_step, in_frame_stride, mask,
+    return run_batch_host_multi(n_devices, devices, width, spacing, in, false, n, rows, cols, in_step, in_frame_stride, mask,
                                 reinterpret_cast<void* const*>(outs), out_step, out_frame_stride, CVS_OUT_F32);
 }
 extern "C" int cvs_g2_run_batch_host_multi_fmt(int n_devices, const int* devices, int width, float spacing, const float* in, int n, int rows,
                                                int cols, size_t in_step, size_t in_frame_stride, unsigned mask, void* const* outs,
                                                size_t out_step, size_t out_frame_stride, int out_format)
 {
-    return run_batch_host_multi(n_devices, devices, width, spacing, in, n, rows, cols, in_step, in_frame_stride, mask, outs, out_step,
+    return run_batch_host_multi(n_devices, devices, width, spacing, in, false, n, rows, cols, in_step, in_frame_stride, mask, outs, out_step,
+                                out_frame_stride, out_format);
+}
+extern "C" int cvs_g2_run_batch_host_multi_u8(int n_devices, const int* devices, int width, float spacing, const uint8_t* in, int n, int rows,
+                                              int cols, size_t in_step, size_t in_frame_stride, unsigned mask, void* const* outs,
+                                              size_t out_step, size_t out_frame_stride, int out_format)
+{
+    return run_batch_host_multi(n_devices, devices, width, spacing, in, true, n, rows, cols, in_step, in_frame_stride, mask, outs, out_step,
                                 out_frame_stride, out_format);
 }
 

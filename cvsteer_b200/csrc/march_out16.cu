@@ -27,8 +27,10 @@ cudaError_t launch_basis_fused16(int family, int fmt, const FamilyTaps& taps, co
 {
     *taken = false;
     if (fmt != 1 && fmt != 2) return cudaErrorInvalidValue;
-    const int px = uses_march_path(family, taps.width) ? out16_kernel_px(family, mask, st.source) : 0;
-    if (!px || g.in_u8 || !tma_eligible(g, family == 2 ? G2Fam::R : G4Fam::R)) return cudaSuccess;
+    // 8-bit frames take the fused kernels where the fp32-output launch would stage them by TMA (march_launch.cuh); the
+    // cooperative `ldg-u8` loader stays on the fallback
+    const int px = uses_march_path(family, taps.width) ? out16_kernel_px(family, mask, st.source, g.in_u8) : 0;
+    if (!px || !tma_eligible(g, family == 2 ? G2Fam::R : G4Fam::R)) return cudaSuccess;
     if (!(family == 2 ? default_taps<G2Fam>(taps) : default_taps<G4Fam>(taps))) return cudaSuccess;
     const int nplanes = family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES;
     const MarchArgs a = make_args(g, mask, st, reinterpret_cast<float* const*>(outs), nplanes);
@@ -48,8 +50,14 @@ cudaError_t launch_basis_fused16(int family, int fmt, const FamilyTaps& taps, co
             ac.theta_map = reinterpret_cast<const float*>(reinterpret_cast<const char*>(a.theta_map) + 2 * (size_t)f0 * g.out_frame_stride);
         if (ac.pyr_out) ac.pyr_out = reinterpret_cast<float*>(reinterpret_cast<char*>(a.pyr_out) + (size_t)f0 * g.next_frame_stride);
         cudaError_t e;
-        if (family == 2)
+        if (family == 2 && g.in_u8)
+            e = fmt == 1 ? launch_march_g2_out16<__half, unsigned char>(taps, gc, ac, stream, info)
+                         : launch_march_g2_out16<__nv_bfloat16, unsigned char>(taps, gc, ac, stream, info);
+        else if (family == 2)
             e = fmt == 1 ? launch_march_g2_out16<__half>(taps, gc, ac, stream, info) : launch_march_g2_out16<__nv_bfloat16>(taps, gc, ac, stream, info);
+        else if (g.in_u8)
+            e = fmt == 1 ? launch_march_g4_out16<__half, unsigned char>(taps, gc, ac, stream, info)
+                         : launch_march_g4_out16<__nv_bfloat16, unsigned char>(taps, gc, ac, stream, info);
         else
             e = fmt == 1 ? launch_march_g4_out16<__half>(taps, gc, ac, stream, info) : launch_march_g4_out16<__nv_bfloat16>(taps, gc, ac, stream, info);
         if (e != cudaSuccess) return e;
@@ -92,6 +100,30 @@ cudaError_t launch_narrow(int fmt, int nplanes, const float* const* src, size_t 
     const dim3 grid((cols + 255) / 256, rows < 65535 ? rows : 65535, n * nplanes);
     if (fmt == 1) k_narrow<__half><<<grid, 256, 0, stream>>>(a);
     else k_narrow<__nv_bfloat16><<<grid, 256, 0, stream>>>(a);
+    g_launches.fetch_add(1);
+    return cudaGetLastError();
+}
+
+// One byte -> fp32 per thread and row (the host-buffer path's 8-bit frames where it must run the fp32-frame kernel).  blockIdx.z
+// and the rows are grid-strided so that any batch fits the grid.
+__global__ void __launch_bounds__(256) k_widen(const unsigned char* src, long long src_pitch, long long src_frame_stride, float* dst,
+                                               long long dst_pitch, long long dst_frame_stride, int n, int rows, int cols)
+{
+    const int x = blockIdx.x * 256 + threadIdx.x;
+    if (x >= cols) return;
+    for (int f = blockIdx.z; f < n; f += gridDim.z)
+        for (int y = blockIdx.y; y < rows; y += gridDim.y)
+            *reinterpret_cast<float*>(reinterpret_cast<char*>(dst) + f * dst_frame_stride + y * dst_pitch + 4ll * x) =
+                (float)src[f * src_frame_stride + y * src_pitch + x];
+}
+
+cudaError_t launch_widen(const unsigned char* src, size_t src_pitch, size_t src_frame_stride, float* dst, size_t dst_pitch,
+                         size_t dst_frame_stride, int n, int rows, int cols, cudaStream_t stream)
+{
+    if (n <= 0 || rows <= 0 || cols <= 0) return cudaErrorInvalidValue;
+    const dim3 grid((cols + 255) / 256, rows < 65535 ? rows : 65535, n < 65535 ? n : 65535);
+    k_widen<<<grid, 256, 0, stream>>>(src, (long long)src_pitch, (long long)src_frame_stride, dst, (long long)dst_pitch,
+                                      (long long)dst_frame_stride, n, rows, cols);
     g_launches.fetch_add(1);
     return cudaGetLastError();
 }

@@ -235,8 +235,9 @@ CVS_API int cvs_g4_run_batch_dev(cvs_g4* h, const cvs_batch* b, unsigned mask, i
  * 2-byte aligned).  The CVS_STEER_MAP angle map stays fp32 in the outputs' ELEMENT layout, so its byte pitch and frame
  * stride are twice the outputs'.  `next_level` stays fp32 and is unchanged (it is the next level's input).
  * Speed: every mask/source pair with a fused kernel above has a fused 16-bit twin (it stores 2 bytes per pixel and plane;
- * two-pixel kernels need 4-byte aligned planes / out_pitch / out_frame_stride).  Everything else -- the cooperative loader,
- * 8-bit input, other taps, other masks, a layout misaligned for the store width -- runs the fp32 kernel into stream-ordered
+ * two-pixel kernels need 4-byte aligned planes / out_pitch / out_frame_stride), for fp32 and for 8-bit input (in_is_u8; one
+ * pixel per thread, TMA-staged: 16-byte aligned `in`, in_pitch and in_frame_stride).  Everything else -- the cooperative
+ * loader, other taps, other masks, a layout misaligned for the store width -- runs the fp32 kernel into stream-ordered
  * scratch on the call's stream and narrows it, with the same bits.  CVS_OUT_F32 is exactly the fp32 call. */
 typedef enum cvs_out_format { CVS_OUT_F32 = 0, CVS_OUT_F16 = 1, CVS_OUT_BF16 = 2 } cvs_out_format;
 CVS_API int cvs_g2_run_batch_dev_fmt(cvs_g2* h, const cvs_batch* b, unsigned mask, int steer_source, float theta_scalar,
@@ -273,6 +274,20 @@ CVS_API int cvs_g4_run_batch_host_fmt(cvs_g4* h, const float* in, int n, int row
                                       unsigned mask, int steer_source, float theta_scalar, void* const* outs, size_t out_step,
                                       size_t out_frame_stride, int out_format);
 
+/* 8-bit host-buffer batches: the arguments of the _fmt calls above, with 8-bit gray frames (`in`, in_step >= cols and
+ * in_frame_stride in bytes of 8-bit rows).  Contract: every plane is, bit for bit, what the fp32-frame call with the same
+ * out_format writes for the same frames widened to float (values 0..255, no scaling); CVS_OUT_F32 is allowed.  A null `in`,
+ * in_step < cols and the 16-bit output layout errors of the _fmt calls are CVS_ERR_INVALID_ARG before the handle is looked at
+ * and before any CUDA call.  Uploads move 1 byte per pixel instead of 4 and the frames stay 8-bit on the device, where the
+ * fused kernels stage them by TMA and widen them in shared memory; dense rows (in_step == cols == a multiple of 128, as
+ * 1920 and 3840 are, in_frame_stride == rows * cols) move as one linear copy per chunk.  With 16-bit planes a caller that
+ * holds 8-bit frames sends 15 bytes per pixel over PCIe for M2 (7 planes) instead of 18, and 7 instead of 10 for M1. */
+CVS_API int cvs_g2_run_batch_host_u8(cvs_g2* h, const uint8_t* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                     unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride, int out_format);
+CVS_API int cvs_g4_run_batch_host_u8(cvs_g4* h, const uint8_t* in, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                     unsigned mask, int steer_source, float theta_scalar, void* const* outs, size_t out_step,
+                                     size_t out_frame_stride, int out_format);
+
 /* ---- the callers' 8-bit post-processing (reference example/steer.cpp:92-104, test/test.cpp:93-95), on the device ----
  * gain > 0: Mat::convertTo(CV_8UC1, gain); gain <= 0: cv::normalize(src, dst, 0, 255, NORM_MINMAX, CV_8UC1), per frame. */
 CVS_API int cvs_to_u8_dev(int device, const float* src, int n, int rows, int cols, size_t pitch, size_t frame_stride, float gain,
@@ -297,6 +312,10 @@ CVS_API int cvs_g2_run_batch_host_multi(int n_devices, const int* devices, int w
 CVS_API int cvs_g2_run_batch_host_multi_fmt(int n_devices, const int* devices, int width, float spacing, const float* in, int n,
                                             int rows, int cols, size_t in_step, size_t in_frame_stride, unsigned mask,
                                             void* const* outs, size_t out_step, size_t out_frame_stride, int out_format);
+/* 8-bit-frame twin of cvs_g2_run_batch_host_multi_fmt (see cvs_g2_run_batch_host_u8) */
+CVS_API int cvs_g2_run_batch_host_multi_u8(int n_devices, const int* devices, int width, float spacing, const uint8_t* in, int n,
+                                           int rows, int cols, size_t in_step, size_t in_frame_stride, unsigned mask,
+                                           void* const* outs, size_t out_step, size_t out_frame_stride, int out_format);
 
 /* The row-band plan both band paths use (this library's multi-GPU entry point below and cvsteer_b200/multi.py), for
  * callers that shard one huge image over one process per GPU themselves.  Band edges sit on multiples of 2^(levels-1)
