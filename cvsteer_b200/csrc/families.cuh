@@ -109,7 +109,7 @@ struct G2Fam {
                 ct = a.cos_t;
                 st = a.sin_t;
             } else if (FAST) {
-                __sincosf(theta_px, &st, &ct);  // MUFU works on theta / 2 pi mod 1: abs error < 5e-7 (+ 6e-8 |theta| beyond pi)
+                __sincosf(theta_px, &st, &ct);  // MUFU works on theta / 2 pi mod 1: abs error < 3.6e-7 (+ 1.6e-7 |theta| beyond pi)
             } else {
                 dev::sincos_steer(theta_px, &st, &ct);
             }
@@ -261,8 +261,8 @@ struct G4Fam {
             ct = ct_pre;
             st = st_pre;
         } else if (FAST) {
-            // MUFU.SIN/COS work on theta / 2 pi modulo 1: no range branch, abs error < 5e-7 for |theta| <= pi and
-            // ~6e-8 * |theta| beyond (the fp32 rounding of theta / 2 pi) -- 1e-6 of the basis range after steering
+            // MUFU.SIN/COS work on theta / 2 pi modulo 1: no range branch, abs error < 3.6e-7 for |theta| <= pi and up to
+            // 1.6e-7 * |theta| more beyond (theta * float(1 / 2 pi) rounds toward zero: < 2u, plus the constant's 0.68u)
             __sincosf(theta_px, &st, &ct);
         } else {
             dev::sincos_steer(theta_px, &st, &ct);
