@@ -81,6 +81,38 @@ def _host_frames(x: torch.Tensor):
     return x.dtype == torch.uint8, x.stride(1) * es, x.stride(0) * es
 
 
+def _bank_angles(thetas, mask: int):
+    """float array of the bank's angles; the angle count and the mask checked before anything touches a device."""
+    th = [float(t) for t in thetas]
+    if not 1 <= len(th) <= capi.BANK_MAX_ANGLES:
+        raise capi.CvsError(capi.ERR_INVALID_ARG, f"a bank steers to 1..{capi.BANK_MAX_ANGLES} angles, got {len(th)}")
+    if not mask or mask & ~capi.G2_BANK_PLANES:
+        raise capi.CvsError(capi.ERR_INVALID_ARG, f"bank mask 0x{mask:x}: bank planes are 0x{capi.G2_BANK_PLANES:x}")
+    return (C.c_float * len(th))(*th)
+
+
+def _bank_layout(outs: Dict[int, torch.Tensor], planes, shape_angle, shape_once):
+    """(out_pitch, out_frame_stride, angle_stride) in bytes shared by the bank's planes: per-angle planes are
+    [N, n, rows, cols] views, theta / strength [n, rows, cols]; any strides with unit column stride."""
+    lay = set()
+    for p in planes:
+        t = outs[p]
+        per_angle = capi.G2_MASK_STEER5 >> p & 1
+        want = shape_angle if per_angle else shape_once
+        if tuple(t.shape) != want or t.stride(-1) != 1:
+            raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"output plane {p}: need {want} with unit column stride, got {tuple(t.shape)}")
+        es = t.element_size()
+        st = [s * es for s in t.stride()]
+        lay.add((st[-2], st[-3], st[0] if per_angle else None))
+    pitches = {l[:2] for l in lay}
+    angle = {l[2] for l in lay if l[2] is not None}
+    if len(pitches) != 1 or len(angle) > 1:
+        raise capi.CvsError(capi.ERR_INVALID_ARG, "the bank's planes share one row pitch and frame stride, and the per-angle "
+                                                  "planes one angle stride")
+    pitch, fstride = pitches.pop()
+    return pitch, fstride, angle.pop() if angle else 0
+
+
 def _stream_ptr(stream):
     s = stream if stream is not None else torch.cuda.current_stream()
     return C.c_void_p(s.cuda_stream)
@@ -210,6 +242,67 @@ class G2Batch(_FusedBatch):
             capi.check(self._lib.cvs_g2_run_batch_host(*args))
         else:
             capi.check(self._lib.cvs_g2_run_batch_host_fmt(*args, fmt))
+
+
+    def steer_bank(self, frames: torch.Tensor, thetas, mask: int = capi.G2_MASK_STEER5, outs: Optional[Dict[int, torch.Tensor]] = None,
+                   out_dtype: torch.dtype = torch.float32, band: Optional[Band] = None, next_level: Optional[torch.Tensor] = None,
+                   stream=None) -> Dict[str, torch.Tensor]:
+        """Steering bank (cvs_g2_steer_bank_dev): one filtering pass, then the planes of `mask` at every angle of `thetas`
+        (1..16 of them).  Returns {name: tensor}: [N, n, out_rows, cols] for the per-angle planes (g2, h2, e, magnitude,
+        phase), [n, out_rows, cols] for theta and strength.  Each per-angle plane k is, bit for bit, that plane of
+        run(frames, G2_MASK_STEER5, STEER_SCALAR, thetas[k]); theta / strength those of run(frames, G2_MASK_ORIENT).
+        outs: optional {plane: tensor} of those shapes with any strides of unit column stride, e.g. a [n, N, rows, cols]
+        tensor seen through .transpose(0, 1); the planes share one row pitch and frame stride.  band and next_level as in run()."""
+        th = _bank_angles(thetas, mask)
+        x = _as_batch(frames)
+        if x.device.index != self.device:
+            raise capi.CvsError(capi.ERR_INVALID_ARG, f"frames live on cuda:{x.device.index}, this handle on cuda:{self.device}")
+        n, rows, cols = x.shape
+        out_rows = rows if band is None else band.row_end - band.row_begin
+        planes = [p for p in range(capi.G2_NPLANES) if mask >> p & 1]
+        fmt = _out_format(out_dtype)
+        shape_angle, shape_once = (len(th), n, out_rows, cols), (n, out_rows, cols)
+        if outs is None:
+            outs = {p: torch.empty(shape_angle if capi.G2_MASK_STEER5 >> p & 1 else shape_once, dtype=out_dtype, device=x.device)
+                    for p in planes}
+        for p in planes:
+            if p not in outs:
+                raise capi.CvsError(capi.ERR_INVALID_ARG, f"no output plane for {p}")
+            if outs[p].dtype != out_dtype or outs[p].device != x.device:
+                raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"output plane {p}: need {out_dtype} on {x.device}")
+        pitch, fstride, astride = _bank_layout(outs, planes, shape_angle, shape_once)
+        arr = (C.c_void_p * capi.G2_NPLANES)()
+        for p in planes:
+            arr[p] = outs[p].data_ptr()
+        b = _batch_struct(x, pitch, fstride, band)
+        if next_level is not None:
+            want = (n, (rows + 1) // 2, (cols + 1) // 2)
+            if tuple(next_level.shape) != want or next_level.dtype != torch.float32 or not next_level.is_contiguous():
+                raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"next_level must be contiguous float32 {want}")
+            b.next_level = next_level.data_ptr()
+            b.next_pitch, b.next_frame_stride = want[2] * 4, want[1] * want[2] * 4
+        with torch.cuda.device(self.device):
+            capi.check(self._lib.cvs_g2_steer_bank_dev(self._h, C.byref(b), th, len(th), mask, arr, astride, _stream_ptr(stream), fmt))
+        return {self._names[p]: outs[p] for p in planes}
+
+    def steer_bank_host(self, frames_host: torch.Tensor, thetas, mask: int, outs_host: Dict[int, torch.Tensor]):
+        """Host-buffer twin of steer_bank (cvs_g2_steer_bank_host): pinned float32 or uint8 frames [n, rows, cols] in, pinned
+        planes out ([N, n, rows, cols] per angle, [n, rows, cols] for theta / strength, one dtype that selects the format)."""
+        th = _bank_angles(thetas, mask)
+        x = frames_host
+        u8, step, fstride = _host_frames(x)
+        n, rows, cols = x.shape
+        fmt, _ = _host_format(outs_host)
+        planes = [p for p in range(capi.G2_NPLANES) if mask >> p & 1]
+        missing = [p for p in planes if p not in outs_host]
+        if missing:
+            raise capi.CvsError(capi.ERR_INVALID_ARG, f"no output plane for {missing}")
+        pitch, ofs, astride = _bank_layout(outs_host, planes, (len(th), n, rows, cols), (n, rows, cols))
+        arr = (C.c_void_p * capi.G2_NPLANES)()
+        for p in planes:
+            arr[p] = outs_host[p].data_ptr()
+        capi.check(self._lib.cvs_g2_steer_bank_host(self._h, C.c_void_p(x.data_ptr()), int(u8), n, rows, cols, step, fstride, th, len(th),
+                                                    mask, arr, pitch, ofs, astride, fmt))
 
 
 class G4Batch(_FusedBatch):

@@ -336,6 +336,57 @@ int run_fused_fmt(Filter* f, const BatchGeom& g, unsigned mask, const SteerSpec&
     return CVS_OK;
 }
 
+// Steering bank (cvs_g2_steer_bank_dev): the fused bank kernel when its forms apply, otherwise the calls the contract names --
+// one STEER5 launch per scalar angle and one ORIENT launch at theta_d when theta_d or strength is wanted -- with the planes they
+// write but the caller did not select in stream-ordered scratch of the caller's layout.  Both give the same bits.
+int run_bank(Filter* f, const BatchGeom& g, const BankSpec& bk, int fmt, cudaStream_t stream, int slot = 0, int nslots = 1)
+{
+    CU_TRY(cudaSetDevice(f->device));
+    bool taken = false;
+    CU_TRY(launch_g2_bank(fmt, f->taps, g, bk, stream, &f->last, &taken));
+    if (taken) return CVS_OK;
+    const unsigned orient_bits = CVS_BIT(CVS_THETA) | CVS_BIT(CVS_STRENGTH);
+    const bool steer = (bk.mask & CVS_G2_MASK_STEER5) != 0, orient = (bk.mask & orient_bits) != 0;
+    unsigned scr = 0;  // planes written to scratch: E of the ORIENT launch always (the caller's E planes hold E(theta_k))
+    if (steer) scr |= CVS_G2_MASK_STEER5 & ~bk.mask;
+    if (orient) scr |= CVS_G2_MASK_ORIENT & ~(bk.mask & orient_bits);
+    const size_t set_bytes = (size_t)(g.n - 1) * g.out_frame_stride + (size_t)(g.out_row_end - g.out_row_begin) * g.out_pitch;
+    void* scratch = nullptr;
+    if (scr) CU_TRY(cudaMallocAsync(&scratch, set_bytes * __builtin_popcount(scr), stream));
+    void* so[CVS_G2_NPLANES] = {nullptr};
+    for (int q = 0, i = 0; q < CVS_G2_NPLANES; ++q)
+        if (scr >> q & 1u) so[q] = static_cast<char*>(scratch) + (size_t)(i++) * set_bytes;
+    auto pick = [&](int q, size_t off) -> void* { return (bk.mask >> q & 1u) ? static_cast<char*>(bk.outs[q]) + off : so[q]; };
+    char first[sizeof(f->last.name)] = "";
+    BatchGeom gk = g;
+    int rc = CVS_OK;
+    for (int k = 0; steer && k < bk.n_angles && rc == CVS_OK; ++k) {
+        void* outs[CVS_G2_NPLANES] = {nullptr};
+        for (int q = 0; q < CVS_G2_NPLANES; ++q)
+            if (CVS_G2_MASK_STEER5 >> q & 1u) outs[q] = pick(q, (size_t)k * bk.angle_stride);
+        SteerSpec st{};
+        st.source = CVS_STEER_SCALAR;
+        st.cos_t = bk.cos_t[k];
+        st.sin_t = bk.sin_t[k];
+        rc = run_fused_fmt(f, gk, CVS_G2_MASK_STEER5, st, outs, fmt, stream, slot, nslots);
+        if (!first[0]) snprintf(first, sizeof(first), "%s", f->last.name);
+        gk.next_level = nullptr;  // the first launch emitted it
+    }
+    if (orient && rc == CVS_OK) {
+        void* outs[CVS_G2_NPLANES] = {nullptr};
+        outs[CVS_THETA] = pick(CVS_THETA, 0), outs[CVS_STRENGTH] = pick(CVS_STRENGTH, 0), outs[CVS_E] = so[CVS_E];
+        SteerSpec st{};
+        st.source = CVS_STEER_DOMINANT;
+        rc = run_fused_fmt(f, gk, CVS_G2_MASK_ORIENT, st, outs, fmt, stream, slot, nslots);
+        if (!first[0]) snprintf(first, sizeof(first), "%s", f->last.name);
+    }
+    const cudaError_t e = scr ? cudaFreeAsync(scratch, stream) : cudaSuccess;
+    if (rc != CVS_OK) return rc;
+    CU_TRY(e);
+    snprintf(f->last.name, sizeof(f->last.name), "bank-fallback:%s", first);
+    return CVS_OK;
+}
+
 int filter_setup(Filter* f, const void* image, bool u8, int rows, int cols, size_t step)
 {
     if (!f) return fail(CVS_ERR_INVALID_ARG, "handle is null");
@@ -710,6 +761,63 @@ extern "C" int cvs_g4_run_batch_dev_fmt(cvs_g4* h, const cvs_batch* b, unsigned 
     return run_batch_dev(reinterpret_cast<Filter*>(h), b, mask, steer_source, theta_scalar, theta_map, outs, stream, out_format);
 }
 
+// Steering-bank arguments, checked before the handle is looked at and before any CUDA call.  out_rows: rows of one output plane.
+static int check_bank(const float* thetas, int n_angles, unsigned mask, void* const* outs, int fmt, int cols, int n, int out_rows, size_t out_pitch,
+                      size_t out_frame_stride, size_t angle_stride)
+{
+    if (n_angles < 1 || n_angles > CVS_BANK_MAX_ANGLES) return fail(CVS_ERR_INVALID_ARG, "n_angles %d outside [1, %d]", n_angles, CVS_BANK_MAX_ANGLES);
+    if (!thetas) return fail(CVS_ERR_INVALID_ARG, "thetas is null");
+    if (!mask || (mask & ~(unsigned)CVS_G2_BANK_PLANES)) return fail(CVS_ERR_INVALID_ARG, "mask 0x%x: bank planes are 0x%x", mask, (unsigned)CVS_G2_BANK_PLANES);
+    if (!outs) return fail(CVS_ERR_INVALID_ARG, "outs is null");
+    for (int p = 0; p < CVS_G2_NPLANES; ++p)
+        if ((mask >> p & 1u) && !outs[p]) return fail(CVS_ERR_INVALID_ARG, "outs[%d] is null but selected by mask", p);
+    if (fmt != CVS_OUT_F32)
+        if (int rc = check_out16(fmt, cols, out_pitch, mask, CVS_G2_NPLANES, outs)) return rc;
+    const size_t esz = fmt == CVS_OUT_F32 ? 4 : 2;
+    if (out_pitch < (size_t)cols * esz) return fail(CVS_ERR_INVALID_ARG, "out_pitch %zu < cols*%zu", out_pitch, esz);
+    if ((out_frame_stride | angle_stride) & (esz - 1))
+        return fail(CVS_ERR_INVALID_ARG, "out_frame_stride %zu / angle_stride %zu not multiples of %zu bytes", out_frame_stride, angle_stride, esz);
+    // no two (angle, frame) planes of one quantity overlap: sort the strides of the dimensions that have more than one plane
+    struct Dim { long long count; size_t stride; } d[2];
+    int nd = 0;
+    if ((mask & CVS_G2_MASK_STEER5) && n_angles > 1) d[nd++] = {n_angles, angle_stride};
+    if (n > 1) d[nd++] = {n, out_frame_stride};
+    if (nd == 2 && d[1].stride < d[0].stride) std::swap(d[0], d[1]);
+    const size_t extent = (size_t)std::max(out_rows, 0) * out_pitch;
+    if ((nd >= 1 && d[0].stride < extent) || (nd == 2 && d[1].stride / (size_t)d[0].count < d[0].stride))
+        return fail(CVS_ERR_INVALID_ARG, "angle_stride %zu and out_frame_stride %zu overlap planes of %zu bytes (%d angles, %d frames)", angle_stride,
+                    out_frame_stride, extent, n_angles, n);
+    return CVS_OK;
+}
+
+static BankSpec make_bank(const float* thetas, int n_angles, unsigned mask, void* const* outs, size_t angle_stride)
+{
+    BankSpec bk{};
+    bk.n_angles = n_angles;
+    bk.mask = mask;
+    for (int k = 0; k < n_angles; ++k) bk.cos_t[k] = std::cos(thetas[k]), bk.sin_t[k] = std::sin(thetas[k]);  // as run_batch_dev
+    for (int p = 0; p < CVS_G2_NPLANES; ++p) bk.outs[p] = (mask >> p & 1u) ? outs[p] : nullptr;
+    bk.angle_stride = angle_stride;
+    return bk;
+}
+
+extern "C" int cvs_g2_steer_bank_dev(cvs_g2* h, const cvs_batch* b, const float* thetas, int n_angles, unsigned mask, void* const* outs,
+                                     size_t angle_stride, void* stream, int out_format)
+{
+    if (!b) return fail(CVS_ERR_INVALID_ARG, "batch is null");
+    const int out_rows = b->full_rows > 0 ? b->out_row_end - b->out_row_begin : b->rows;
+    if (int rc = check_bank(thetas, n_angles, mask, outs, out_format, b->cols, b->n, out_rows, b->out_pitch, b->out_frame_stride, angle_stride))
+        return rc;
+    Filter* f = reinterpret_cast<Filter*>(h);
+    if (!f || f->family != 2) return fail(CVS_ERR_INVALID_ARG, "handle is null or not a G2 handle");
+    BatchGeom g;
+    int rc = geom_from_batch(b, &g, out_format == CVS_OUT_F32 ? 4 : 2);
+    if (rc) return rc;
+    rc = check_band(g, f->taps.width, g.full_rows);
+    if (rc) return rc;
+    return run_bank(f, g, make_bank(thetas, n_angles, mask, outs, angle_stride), out_format, static_cast<cudaStream_t>(stream));
+}
+
 extern "C" int cvs_pyr_down_dev(int device, const cvs_batch* b, float* out, void* stream)
 {
     BatchGeom g;
@@ -742,8 +850,11 @@ int check_in_u8(const void* in, int cols, size_t in_step)
 
 // in_u8: 8-bit frames (in_step / in_frame_stride in bytes of them), else fp32; the device holds them in the same element type.
 // fmt: cvs_out_format of the host output planes (out_step / out_frame_stride in bytes of them)
+// bank: a steering bank (G2) instead of one launch of `mask` -- its mask and host planes are `mask` / `outs`, per-angle plane p of
+// angle k at outs[p] + k * bank->angle_stride; each (plane, angle) pair is one more device plane per chunk and one more download
 int run_batch_host(Filter* f, int family, const void* in, bool in_u8, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
-                   unsigned mask, int steer_source, float theta, void* const* outs, size_t out_step, size_t out_frame_stride, int fmt = CVS_OUT_F32)
+                   unsigned mask, int steer_source, float theta, void* const* outs, size_t out_step, size_t out_frame_stride, int fmt = CVS_OUT_F32,
+                   const BankSpec* bank = nullptr)
 {
     const size_t esz = fmt == CVS_OUT_F32 ? 4 : 2, in_esz = in_u8 ? 1 : 4;
     if (in_u8)
@@ -760,11 +871,13 @@ int run_batch_host(Filter* f, int family, const void* in, bool in_u8, int n, int
     if (in_step < (size_t)cols * in_esz) return fail(CVS_ERR_INVALID_ARG, "in_step < cols*%zu", in_esz);
     if (out_step < (size_t)cols * esz) return fail(CVS_ERR_INVALID_ARG, "step < cols*%zu", esz);
     if (!mask || (mask >> NPLANES)) return fail(CVS_ERR_INVALID_ARG, "mask 0x%x", mask);
+    // device planes per frame: one per selected plane, or one per angle for a bank's per-angle planes
+    auto copies = [&](int p) { return bank && (CVS_G2_MASK_STEER5 >> p & 1u) ? bank->n_angles : 1; };
     int nout = 0;
     for (int p = 0; p < NPLANES; ++p)
         if (mask >> p & 1u) {
             if (!outs[p]) return fail(CVS_ERR_INVALID_ARG, "outs[%d] is null but selected by mask", p);
-            ++nout;
+            nout += copies(p);
         }
     CU_TRY(cudaSetDevice(f->device));
     const size_t in_row = (size_t)cols * in_esz, pitch = align_up(in_row, 128), fbytes = pitch * rows;  // device input frames
@@ -822,32 +935,41 @@ int run_batch_host(Filter* f, int family, const void* in, bool in_u8, int n, int
         void* douts[(int)CVS_G2_NPLANES > (int)CVS_G4_NPLANES ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES] = {nullptr};
         int slot = 0;
         for (int p = 0; p < NPLANES; ++p)
-            if (mask >> p & 1u) douts[p] = base + (size_t)chunk * fbytes + (size_t)(slot++) * chunk * obytes;
+            if (mask >> p & 1u) douts[p] = base + (size_t)chunk * fbytes + (size_t)slot * chunk * obytes, slot += copies(p);
         BatchGeom g = whole_frame_geom(din, in_u8, nf, rows, cols, pitch, fbytes, opitch, obytes);
         if (widen) {
             float* dw = reinterpret_cast<float*>(base + (size_t)chunk * (fbytes + nout * obytes));
             CU_TRY(launch_widen(reinterpret_cast<const unsigned char*>(din), pitch, fbytes, dw, wpitch, wbytes, nf, rows, cols, s));
             g = whole_frame_geom(dw, false, nf, rows, cols, wpitch, wbytes, opitch, obytes);
         }
-        int rc = run_fused_fmt(f, g, mask, st, douts, fmt, s, b, NBUF);
+        int rc;
+        if (bank) {  // on the device, angle k of a per-angle plane follows the chunk's frames of angle k - 1
+            BankSpec bd = *bank;
+            for (int p = 0; p < NPLANES; ++p) bd.outs[p] = douts[p];
+            bd.angle_stride = (size_t)chunk * obytes;
+            rc = run_bank(f, g, bd, fmt, s, b, NBUF);
+        } else {
+            rc = run_fused_fmt(f, g, mask, st, douts, fmt, s, b, NBUF);
+        }
         if (rc) return rc;
         const size_t row_bytes = (size_t)cols * esz;
         for (int p = 0; p < NPLANES; ++p)
-            if (mask >> p & 1u) {
-                char* dst = static_cast<char*>(outs[p]) + (size_t)f0 * out_frame_stride;
+            for (int a = 0; (mask >> p & 1u) && a < copies(p); ++a) {
+                char* dst = static_cast<char*>(outs[p]) + (size_t)f0 * out_frame_stride + (size_t)a * (bank ? bank->angle_stride : 0);
+                char* src = static_cast<char*>(douts[p]) + (size_t)a * chunk * obytes;
                 if (opitch == row_bytes && out_step == opitch && out_frame_stride == obytes) {
-                    CU_TRY(cudaMemcpyAsync(dst, douts[p], (size_t)nf * obytes, cudaMemcpyDeviceToHost, s));
+                    CU_TRY(cudaMemcpyAsync(dst, src, (size_t)nf * obytes, cudaMemcpyDeviceToHost, s));
                 } else if (out_frame_stride % out_step == 0) {
                     cudaMemcpy3DParms cq{};
-                    cq.srcPtr = make_cudaPitchedPtr(douts[p], opitch, row_bytes, rows);
+                    cq.srcPtr = make_cudaPitchedPtr(src, opitch, row_bytes, rows);
                     cq.dstPtr = make_cudaPitchedPtr(dst, out_step, row_bytes, out_frame_stride / out_step);
                     cq.extent = make_cudaExtent(row_bytes, rows, nf);
                     cq.kind = cudaMemcpyDeviceToHost;
                     CU_TRY(cudaMemcpy3DAsync(&cq, s));
                 } else {
                     for (int k = 0; k < nf; ++k)
-                        CU_TRY(cudaMemcpy2DAsync(dst + (size_t)k * out_frame_stride, out_step, static_cast<char*>(douts[p]) + (size_t)k * obytes,
-                                                 opitch, row_bytes, rows, cudaMemcpyDeviceToHost, s));
+                        CU_TRY(cudaMemcpy2DAsync(dst + (size_t)k * out_frame_stride, out_step, src + (size_t)k * obytes, opitch, row_bytes, rows,
+                                                 cudaMemcpyDeviceToHost, s));
                 }
             }
     }
@@ -894,6 +1016,19 @@ extern "C" int cvs_g4_run_batch_host_u8(cvs_g4* h, const uint8_t* in, int n, int
 {
     return run_batch_host(reinterpret_cast<Filter*>(h), 4, in, true, n, rows, cols, in_step, in_frame_stride, mask, steer_source, theta_scalar, outs,
                           out_step, out_frame_stride, out_format);
+}
+
+extern "C" int cvs_g2_steer_bank_host(cvs_g2* h, const void* in, int in_is_u8, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                      const float* thetas, int n_angles, unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride,
+                                      size_t angle_stride, int out_format)
+{
+    if (int rc = check_bank(thetas, n_angles, mask, outs, out_format, cols, n, rows, out_step, out_frame_stride, angle_stride)) return rc;
+    if (!in) return fail(CVS_ERR_INVALID_ARG, "in is null");
+    const size_t in_esz = in_is_u8 ? 1 : 4;
+    if (in_step < (size_t)cols * in_esz) return fail(CVS_ERR_INVALID_ARG, "in_step %zu < cols*%zu", in_step, in_esz);
+    const BankSpec bk = make_bank(thetas, n_angles, mask, outs, angle_stride);
+    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, in_is_u8 != 0, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_SCALAR, 0.f, outs,
+                          out_step, out_frame_stride, out_format, &bk);
 }
 
 extern "C" int cvs_to_u8_dev(int device, const float* src, int n, int rows, int cols, size_t pitch, size_t frame_stride, float gain, uint8_t* dst,

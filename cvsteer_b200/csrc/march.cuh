@@ -467,10 +467,11 @@ __device__ __forceinline__ void emit_next_level(const float* tile, const MarchAr
 // shared-memory loads (K + 1 values as 8-byte loads feed two pixels instead of K values feeding one), store instructions
 // and their 64-bit address arithmetic (one 8-byte store per plane for two pixels), loop control.
 // TOut: element type of the output planes (float, or __half / __nv_bfloat16 rounded at the store; see OutCursor).
-template <class Fam, unsigned MASK /* 0 = use a.mask at run time */, bool USE_TMA, typename TIn, bool BAKED, int PX = 1, typename TOut = float>
-__global__ void __launch_bounds__(MARCH_TW / PX, (PX == 2 && CVS_PX2_MIN_CTAS > 0) ? CVS_PX2_MIN_CTAS : Fam::MIN_CTAS)
-k_march(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ MarchArgs a,
-        const __grid_constant__ TapTable<Fam::NSETS, Fam::R> taps)
+// march_body is the whole kernel; the epilogue stores through a Cursor(out, band_off, x) (k_march: an OutCursor on a.out[], with
+// out = a; k_bank in march_bank.cuh: the bank's per-angle planes).
+template <class Fam, unsigned MASK, bool USE_TMA, typename TIn, bool BAKED, int PX, typename TOut, class Cursor, class OutArgs>
+__device__ __forceinline__ void march_body(const CUtensorMap& tmap, const MarchArgs& a, const TapTable<Fam::NSETS, Fam::R>& taps,
+                                           const OutArgs& out)
 {
     constexpr int R = Fam::R, K = 2 * R + 1, TW = MARCH_TW, TWH = march_tile_width(R), BH = Fam::BH, TROWS = BH + 2 * R;
     constexpr int NROW = Fam::NROW, NB = Fam::NBASIS, NT = TW / PX;
@@ -644,10 +645,7 @@ k_march(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ MarchA
     // the price of NROW register moves per row): this is what keeps the loop body inside the instruction cache.
     // Output addressing: see OutCursor.
     const long long band_off = (long long)frame * a.out_frame_stride + (long long)(yb - a.out_row_origin) * a.out_pitch;
-    // per-plane base registers only pay off while there are few planes (2 registers each); wide masks share one offset
-    // (the same goes for the families whose nine 13-row windows leave no registers to spare: G4)
-    using Cursor = OutCursor<((__builtin_popcount(MASK & MARCH_PLANE_BITS) <= CVS_CURSOR_MAX_PLANES && !Fam::SHARED_ROW_PASS) ? MASK : 0u), Fam::NPLANES, TOut>;
-    Cursor cur(a, band_off, x);
+    Cursor cur(out, band_off, x);
     // point-wise epilogue of the row just finished by col_pass (+ the stores), then on to the next output row
     auto emit_row = [&](float th, float th_right = 0.f) {  // th_right: the right pixel's steering angle (two-pixel @map kernels)
         if constexpr (PX == 1) {
@@ -889,6 +887,17 @@ k_march(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ MarchA
         }
     }
     if (a.pyr_out) emit_next_level<R, BH, NT>(tile, a, frame, x0, yb);  // CTA-uniform; the tile is read-only after staging
+}
+
+template <class Fam, unsigned MASK /* 0 = use a.mask at run time */, bool USE_TMA, typename TIn, bool BAKED, int PX = 1, typename TOut = float>
+__global__ void __launch_bounds__(MARCH_TW / PX, (PX == 2 && CVS_PX2_MIN_CTAS > 0) ? CVS_PX2_MIN_CTAS : Fam::MIN_CTAS)
+k_march(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ MarchArgs a,
+        const __grid_constant__ TapTable<Fam::NSETS, Fam::R> taps)
+{
+    // per-plane base registers only pay off while there are few planes (2 registers each); wide masks share one offset
+    // (the same goes for the families whose nine 13-row windows leave no registers to spare: G4)
+    using Cursor = OutCursor<((__builtin_popcount(MASK & MARCH_PLANE_BITS) <= CVS_CURSOR_MAX_PLANES && !Fam::SHARED_ROW_PASS) ? MASK : 0u), Fam::NPLANES, TOut>;
+    march_body<Fam, MASK, USE_TMA, TIn, BAKED, PX, TOut, Cursor>(tmap, a, taps, a);
 }
 
 }  // namespace cvs

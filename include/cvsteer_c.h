@@ -288,6 +288,39 @@ CVS_API int cvs_g4_run_batch_host_u8(cvs_g4* h, const uint8_t* in, int n, int ro
                                      unsigned mask, int steer_source, float theta_scalar, void* const* outs, size_t out_step,
                                      size_t out_frame_stride, int out_format);
 
+/* ---- steering banks: one filtering pass, the steered planes at up to 16 angles ----
+ * The basis is filtered once per pixel and steered to each of `n_angles` scalar angles thetas[k] (a host array) in the same
+ * launch: an oriented-energy or texture feature bank, or one level of a steerable pyramid, without re-reading the frames.
+ * Bits of `mask`: per angle any of CVS_G2T, CVS_H2T, CVS_E, CVS_MAG, CVS_PHASE; once per pixel CVS_THETA, CVS_STRENGTH.
+ * Layout (bytes): angle k of frame f of per-angle plane p at  outs[p] + k*angle_stride + f*out_frame_stride + row*out_pitch;
+ * theta_d and strength at  outs[p] + f*out_frame_stride + row*out_pitch.  angle_stride and out_frame_stride may come in
+ * either order ([N, n, rows, cols] or [n, N, rows, cols] tensors), but no two (angle, frame) planes of one quantity may
+ * overlap: the smaller stride must be at least one plane (output rows x out_pitch) and the larger must span all the
+ * planes of the smaller.  A count of 1 (one frame, one angle, or no per-angle plane) puts no condition on its stride.
+ * Contract, for fp32 and 8-bit frames and every out_format:
+ *   - for every k, each selected per-angle plane equals, bit for bit, that plane of
+ *     cvs_g2_run_batch_dev_fmt(h, b, CVS_G2_MASK_STEER5, CVS_STEER_SCALAR, thetas[k], ..., out_format);
+ *   - theta_d and strength equal, bit for bit, those of CVS_G2_MASK_ORIENT at CVS_STEER_DOMINANT.
+ * The band fields of `b` and next_level are honoured as in cvs_g2_run_batch_dev.  Argument errors are CVS_ERR_INVALID_ARG
+ * before the handle is looked at and before any CUDA call: n_angles outside [1, CVS_BANK_MAX_ANGLES] or null thetas, mask
+ * bits outside CVS_G2_BANK_PLANES or none, a null selected plane, an unknown out_format and the 16-bit layout rules of the
+ * _fmt calls (angle_stride included), overlapping planes, and (host call) in_step below cols times the element size.
+ * Speed: with the default width and taps, TMA-eligible frames (see cvs_g2_run_batch_dev) and planes, pitch and strides
+ * aligned to the element size, the whole batch is one fused launch (cvs_g2_last_launch: g2_bank/...).  Anything else runs
+ * the calls the contract names, one per angle plus one CVS_G2_MASK_ORIENT launch for theta_d / strength, with unselected
+ * quantities in stream-ordered scratch (bank-fallback:<the per-angle kernel>).  More than 16 angles: split the list. */
+#define CVS_BANK_MAX_ANGLES 16
+#define CVS_G2_BANK_PLANES (CVS_G2_MASK_STEER5 | CVS_BIT(CVS_THETA) | CVS_BIT(CVS_STRENGTH))
+CVS_API int cvs_g2_steer_bank_dev(cvs_g2* h, const cvs_batch* b, const float* thetas /* host, n_angles */, int n_angles, unsigned mask,
+                                  void* const* outs, size_t angle_stride, void* stream, int out_format);
+/* Host-buffer twin (pinned host frames and planes; the chunked upload / kernel / download pipeline of
+ * cvs_g2_run_batch_host_fmt).  in_is_u8: 8-bit frames (in_step / in_frame_stride in bytes of them), else fp32.
+ * Per-angle plane p of angle k, frame f at  outs[p] + k*angle_stride + f*out_frame_stride + row*out_step. */
+CVS_API int cvs_g2_steer_bank_host(cvs_g2* h, const void* in, int in_is_u8, int n, int rows, int cols, size_t in_step,
+                                   size_t in_frame_stride, const float* thetas, int n_angles, unsigned mask,
+                                   void* const* outs, size_t out_step, size_t out_frame_stride, size_t angle_stride,
+                                   int out_format);
+
 /* ---- the callers' 8-bit post-processing (reference example/steer.cpp:92-104, test/test.cpp:93-95), on the device ----
  * gain > 0: Mat::convertTo(CV_8UC1, gain); gain <= 0: cv::normalize(src, dst, 0, 255, NORM_MINMAX, CV_8UC1), per frame. */
 CVS_API int cvs_to_u8_dev(int device, const float* src, int n, int rows, int cols, size_t pitch, size_t frame_stride, float gain,
