@@ -102,9 +102,6 @@ static cudaError_t launch_generic(const FamilyTaps& ft, const BatchGeom& g, cons
     return cudaGetLastError();
 }
 
-cudaError_t launch_march_g2(const FamilyTaps&, const BatchGeom&, const MarchArgs&, bool dominant, cudaStream_t, LaunchInfo*);
-cudaError_t launch_march_g4(const FamilyTaps&, const BatchGeom&, const MarchArgs&, bool dominant, cudaStream_t, LaunchInfo*);
-
 bool uses_march_path(int family, int width) { return (family == 2 && width == G2Fam::R) || (family == 4 && width == G4Fam::R); }
 
 size_t scratch_bytes_generic(int family, const BatchGeom& g)
@@ -131,23 +128,23 @@ cudaError_t launch_basis_fused(int family, const FamilyTaps& taps, const BatchGe
         }
         return e;
     }
-    // gridDim.z carries the frame index: batches beyond 65535 frames go out as several launches
-    for (int f0 = 0; f0 < g.n; f0 += 65535) {
-        BatchGeom gc = g;
-        MarchArgs ac = a;
-        gc.n = g.n - f0 < 65535 ? g.n - f0 : 65535;
-        gc.in = static_cast<const char*>(g.in) + (size_t)f0 * g.in_frame_stride;
-        ac.in = gc.in;
-        for (int p = 0; p < MARCH_MAX_OUT; ++p)
-            if (ac.out[p]) ac.out[p] = reinterpret_cast<float*>(reinterpret_cast<char*>(a.out[p]) + (size_t)f0 * g.out_frame_stride);
-        if (ac.theta_map) ac.theta_map = reinterpret_cast<const float*>(reinterpret_cast<const char*>(a.theta_map) + (size_t)f0 * g.out_frame_stride);
-        if (ac.pyr_out) ac.pyr_out = reinterpret_cast<float*>(reinterpret_cast<char*>(a.pyr_out) + (size_t)f0 * g.next_frame_stride);
-        if (ac.minmax) ac.minmax = a.minmax + 2 * (size_t)f0;
-        const cudaError_t e = family == 2 ? launch_march_g2(taps, gc, ac, st.source == CVS_STEER_DOMINANT, stream, info)
-                                          : launch_march_g4(taps, gc, ac, st.source == CVS_STEER_DOMINANT, stream, info);
-        if (e != cudaSuccess) return e;
-    }
-    return cudaSuccess;
+    bool taken;
+    return family == 2 ? launch_march<G2Fam, float>(taps, g, a, stream, info, &taken) : launch_march<G4Fam, float>(taps, g, a, stream, info, &taken);
+}
+
+cudaError_t launch_basis_fused16(int family, int fmt, const FamilyTaps& taps, const BatchGeom& g, unsigned mask, const SteerSpec& st,
+                                 void* const* outs, cudaStream_t stream, LaunchInfo* info, bool* taken)
+{
+    *taken = false;
+    if (fmt != CVS_OUT_F16 && fmt != CVS_OUT_BF16) return cudaErrorInvalidValue;
+    if (!uses_march_path(family, taps.width)) return cudaSuccess;
+    const int nplanes = family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES;
+    const MarchArgs a = make_args(g, mask, st, reinterpret_cast<float* const*>(outs), nplanes);
+    if (family == 2)
+        return fmt == CVS_OUT_F16 ? launch_march<G2Fam, __half>(taps, g, a, stream, info, taken)
+                                  : launch_march<G2Fam, __nv_bfloat16>(taps, g, a, stream, info, taken);
+    return fmt == CVS_OUT_F16 ? launch_march<G4Fam, __half>(taps, g, a, stream, info, taken)
+                              : launch_march<G4Fam, __nv_bfloat16>(taps, g, a, stream, info, taken);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -451,9 +448,8 @@ cudaError_t launch_pyr_down(const BatchGeom& g, float* out, cudaStream_t stream)
     const int out_rows = g.out_row_end - g.out_row_begin;
     if (out_rows <= 0 || g.n <= 0 || g.n > 65535) return cudaErrorInvalidValue;
     const dim3 grid((out_cols + 127) / 128, out_rows, g.n);
-    static const bool force_simple = getenv("CVS_PYR_SIMPLE") != nullptr;
     // float2 loads need 8-byte aligned rows; every output pitch must be a multiple of 4 bytes (it is: fp32 planes)
-    const bool vec_ok = !g.in_u8 && !force_simple && (((uintptr_t)g.in | g.in_pitch | g.in_frame_stride) & 7) == 0;
+    const bool vec_ok = !g.in_u8 && (((uintptr_t)g.in | g.in_pitch | g.in_frame_stride) & 7) == 0;
     if (vec_ok)
         k_pyr_down_march<<<dim3((out_cols + PD_THREADS - 1) / PD_THREADS, (out_rows + PD_ROWS - 1) / PD_ROWS, g.n), PD_THREADS, 0, stream>>>(
             a, out, out_cols);

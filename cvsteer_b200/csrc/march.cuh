@@ -36,17 +36,10 @@
 // The slot dispatch of the rolled loops is a balanced compare tree, not a switch (which nvcc lowers to a constant-memory
 // jump table: LDC + BRX on the critical path of every row; measured 9-15 % slower).
 // masks with at most this many planes keep a 64-bit base per plane in registers (2 registers each)
-// Two pixels per thread (see k_march's PX): 0 = nowhere, 1 = the M2 kernel (default), 2 = M1 as well.
-// 198 instead of 217 instructions per pixel-row, but with the K-fold unrolled body the loop grows to 57 KB and falls out of
-// the instruction cache (M2 138.9 -> 118.6 Gpix/s); it pays together with the shift loop below (27 KB body, 209
-// instructions per pixel-row): M2 138.9 -> 143.2 Gpix/s at 1080p, 134.7 -> 139.7 at 4K.  M1 (short epilogue) loses 1-2 %
-// that way, so it keeps the unrolled one-pixel kernel.
-#ifndef CVS_MARCH_PX2
-#define CVS_MARCH_PX2 1
-#endif
-// With two-pixel threads: replace the K-fold unrolled body by a "shift" loop -- U row bodies on a LINEAR register window
-// (2R old rows + U new ones), then 2R x NROW x PX register moves shift the window down by U.  Body = U x 2 x ~200
-// instructions (U = 4: 27 KB, inside the instruction cache) at the price of 2R*NROW/U moves per pixel-row.  0 = off.
+// With two-pixel threads (the forms that march_launch.cuh's table gives two pixels): replace the K-fold unrolled body by a
+// "shift" loop -- U row bodies on a LINEAR register window (2R old rows + U new ones), then 2R x NROW x PX register moves
+// shift the window down by U.  Body = U x 2 x ~200 instructions (U = 4: 27 KB, inside the instruction cache) at the price
+// of 2R*NROW/U moves per pixel-row.  0 = off.
 #ifndef CVS_MARCH_SHIFT_U
 #define CVS_MARCH_SHIFT_U 4
 #endif

@@ -1,36 +1,10 @@
-// G2/H2 instantiations of the marching kernel (reference cvsteer/SteerableFiltersG2.cpp:60-177 fused).
-#include "march_launch.cuh"
+// G2/H2 fused kernels with fp32 planes (reference cvsteer/SteerableFiltersG2.cpp:60-177 fused): the run-time-mask
+// kernel, M0, M1 and M2 (march_launch.cuh's G2 table, entries 0-3).
+#include "march_forms.cuh"
 
 namespace cvs {
-
-// march_g2_lines.cu (its own translation unit so that `make -j` compiles it in parallel)
-cudaError_t launch_march_g2_lines(const BatchGeom& g, const MarchArgs& a, const TapTable<G2Fam::NSETS, G2Fam::R>& tt, dim3 grid, cudaStream_t stream,
-                                  LaunchInfo* info);
-
-// march_g2_steer2.cu: the M2 and `lines` masks steered at a scalar angle / an angle map instead of theta_d
-cudaError_t launch_march_g2_given_angle(const BatchGeom& g, const MarchArgs& a, const TapTable<G2Fam::NSETS, G2Fam::R>& tt, dim3 grid, cudaStream_t stream,
-                                        LaunchInfo* info);
-// march_g2_steer.cu: the steer(theta, 5 outputs) mask at a scalar angle / an angle map
-cudaError_t launch_march_g2_steer5(const BatchGeom& g, const MarchArgs& a, const TapTable<G2Fam::NSETS, G2Fam::R>& tt, dim3 grid, cudaStream_t stream,
-                                   LaunchInfo* info);
-
-cudaError_t launch_march_g2(const FamilyTaps& taps, const BatchGeom& g, const MarchArgs& a, bool dom, cudaStream_t stream, LaunchInfo* info)
-{
-    TapTable<G2Fam::NSETS, G2Fam::R> tt;
-    fill_tap_table<G2Fam>(taps, tt);
-    const int out_rows = g.out_row_end - g.out_row_begin;
-    const dim3 grid((g.cols + MARCH_TW - 1) / MARCH_TW, (out_rows + G2Fam::BH - 1) / G2Fam::BH, g.n);
-    const unsigned mask = a.mask;
-    if (dom && mask == CVS_G2_MASK_ORIENT) return launch_march_mask<G2Fam, CVS_G2_MASK_ORIENT, true, (CVS_MARCH_PX2 > 1)>(g, a, tt, grid, stream, info, "g2_march<M1>");
-    if (dom && mask == CVS_G2_MASK_FULL) return launch_march_mask<G2Fam, CVS_G2_MASK_FULL, true, (CVS_MARCH_PX2 > 0)>(g, a, tt, grid, stream, info, "g2_march<M2>");
-    if (mask == CVS_G2_MASK_STATE /* no steered plane: the source is irrelevant */) return launch_march_mask<G2Fam, CVS_G2_MASK_STATE, true>(g, a, tt, grid, stream, info, "g2_march<M0>");
-    static const bool no_lines = getenv("CVS_NO_STATIC_LINES") != nullptr;  // A/B switch
-    if (dom && mask == CVS_G2_MASK_LINES && !no_lines) return launch_march_g2_lines(g, a, tt, grid, stream, info);
-    if (a.minmax) return cudaErrorNotSupported;  // fused min/max statistics exist for the static `lines` kernel only
-    static const bool no_steer5 = getenv("CVS_NO_STATIC_STEER5") != nullptr;  // A/B switch
-    if (!dom && mask == CVS_G2_MASK_STEER5 && !no_steer5) return launch_march_g2_steer5(g, a, tt, grid, stream, info);
-    if (!dom && (mask == CVS_G2_MASK_FULL || mask == CVS_G2_MASK_LINES) && !no_steer5) return launch_march_g2_given_angle(g, a, tt, grid, stream, info);
-    return launch_march_mask<G2Fam, 0u>(g, a, tt, grid, stream, info, "g2_march<dyn>");
-}
-
+CVS_FORM_F32(G2Fam, 0)
+CVS_FORM_F32(G2Fam, 1)
+CVS_FORM_F32(G2Fam, 2)
+CVS_FORM_F32(G2Fam, 3)
 }  // namespace cvs

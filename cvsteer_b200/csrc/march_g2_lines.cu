@@ -1,16 +1,8 @@
-// G2/H2 marching kernel specialised for the cvsteer-run outputs: edges / dark lines / bright lines at theta_d
-// (reference example/steer.cpp:73-90 = SteerableFiltersG2 ctor + steer(theta_d) + find* fused; 16 B/px).
-#include "march_launch.cuh"
+// G2/H2 fused kernels with fp32 planes: edges / dark lines / bright lines at theta_d, without and with the fused
+// min / max statistics (reference example/steer.cpp:73-90; entries 4-5).
+#include "march_forms.cuh"
 
 namespace cvs {
-
-cudaError_t launch_march_g2_lines(const BatchGeom& g, const MarchArgs& a, const TapTable<G2Fam::NSETS, G2Fam::R>& tt, dim3 grid, cudaStream_t stream,
-                                  LaunchInfo* info)
-{
-    if (a.minmax)  // + per-frame min / max of the three maps (cv::normalize NORM_MINMAX statistics) from the same launch
-        return launch_march_mask<G2Fam, CVS_G2_MASK_LINES | MARCH_MINMAX_FLAG, true, (CVS_MARCH_PX2 > 0)>(g, a, tt, grid, stream, info,
-                                                                                                        "g2_march<lines+minmax>");
-    return launch_march_mask<G2Fam, CVS_G2_MASK_LINES, true, (CVS_MARCH_PX2 > 0)>(g, a, tt, grid, stream, info, "g2_march<lines>");
-}
-
+CVS_FORM_F32(G2Fam, 4)
+CVS_FORM_F32(G2Fam, 5)
 }  // namespace cvs

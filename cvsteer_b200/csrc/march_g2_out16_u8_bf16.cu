@@ -1,6 +1,18 @@
-// G2 fused kernels with 8-bit input and bf16 output planes (see march_out16.cuh).
-#include "march_out16.cuh"
+// G2/H2 fused kernels with bf16 planes from 8-bit frames (every G2 entry; those without a 16-bit twin compile to no
+// kernel).
+#include "march_forms.cuh"
 
 namespace cvs {
-template cudaError_t launch_march_g2_out16<__nv_bfloat16, unsigned char>(const FamilyTaps&, const BatchGeom&, const MarchArgs&, cudaStream_t, LaunchInfo*);
+CVS_FORM(G2Fam, 0, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 1, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 2, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 3, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 4, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 5, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 6, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 7, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 8, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 9, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 10, __nv_bfloat16, unsigned char)
+CVS_FORM(G2Fam, 11, __nv_bfloat16, unsigned char)
 }  // namespace cvs

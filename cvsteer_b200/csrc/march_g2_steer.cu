@@ -1,17 +1,8 @@
-// G2/H2 marching kernel specialised for steer(theta, g2, h2, e, magnitude, phase) at a GIVEN angle -- one scalar angle
-// for the whole batch or a per-pixel angle map (reference cvsteer/SteerableFiltersG2.cpp:157-165 and :167-177 fused with the
-// basis stage; 24 / 28 B/px).  Without these, every non-dominant steering request fell into the run-time-mask kernel.
-#include "march_launch.cuh"
+// G2/H2 fused kernels with fp32 planes: steer(theta, g2, h2, e, magnitude, phase) at a scalar angle and at an angle
+// map (reference cvsteer/SteerableFiltersG2.cpp:157-177 fused with the basis stage; entries 6-7).
+#include "march_forms.cuh"
 
 namespace cvs {
-
-cudaError_t launch_march_g2_steer5(const BatchGeom& g, const MarchArgs& a, const TapTable<G2Fam::NSETS, G2Fam::R>& tt, dim3 grid, cudaStream_t stream,
-                                   LaunchInfo* info)
-{
-    if (a.steer_source == CVS_STEER_SCALAR)
-        return launch_march_mask<G2Fam, march_key(CVS_G2_MASK_STEER5, CVS_STEER_SCALAR), true, (CVS_MARCH_PX2 > 0)>(g, a, tt, grid, stream, info,
-                                                                                                                  "g2_march<steer5@scalar>");
-    return launch_march_mask<G2Fam, march_key(CVS_G2_MASK_STEER5, CVS_STEER_MAP), true, (CVS_MARCH_PX2 > 0)>(g, a, tt, grid, stream, info, "g2_march<steer5@map>");
-}
-
+CVS_FORM_F32(G2Fam, 6)
+CVS_FORM_F32(G2Fam, 7)
 }  // namespace cvs

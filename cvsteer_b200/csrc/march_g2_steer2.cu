@@ -1,26 +1,10 @@
-// G2/H2 marching kernel: the M2 mask (theta_d, strength + g2, h2, e, magnitude, phase) and the `lines` mask (edges / dark
-// lines / bright lines) steered at a GIVEN angle -- one scalar or a per-pixel map -- instead of the in-kernel theta_d.
-// With these every steering source of every mask named in include/cvsteer_c.h has a static specialisation; only
-// arbitrary plane combinations still take the run-time-mask kernel.
-#include "march_launch.cuh"
+// G2/H2 fused kernels with fp32 planes: the M2 and `lines` masks steered at a scalar angle and at an angle map instead
+// of theta_d (entries 8-11).
+#include "march_forms.cuh"
 
 namespace cvs {
-
-cudaError_t launch_march_g2_given_angle(const BatchGeom& g, const MarchArgs& a, const TapTable<G2Fam::NSETS, G2Fam::R>& tt, dim3 grid, cudaStream_t stream,
-                                        LaunchInfo* info)
-{
-    const bool scalar = a.steer_source == CVS_STEER_SCALAR;
-    if (a.mask == CVS_G2_MASK_FULL) {
-        if (scalar)
-            return launch_march_mask<G2Fam, march_key(CVS_G2_MASK_FULL, CVS_STEER_SCALAR), true, (CVS_MARCH_PX2 > 0)>(g, a, tt, grid, stream, info,
-                                                                                                                    "g2_march<M2@scalar>");
-        return launch_march_mask<G2Fam, march_key(CVS_G2_MASK_FULL, CVS_STEER_MAP), true, (CVS_MARCH_PX2 > 0)>(g, a, tt, grid, stream, info, "g2_march<M2@map>");
-    }
-    if (scalar)
-        return launch_march_mask<G2Fam, march_key(CVS_G2_MASK_LINES, CVS_STEER_SCALAR), true, (CVS_MARCH_PX2 > 0)>(g, a, tt, grid, stream, info,
-                                                                                                                 "g2_march<lines@scalar>");
-    // (one pixel per thread: measured 152-155 Gpix/s against 142-149 for the two-pixel form of this mask)
-    return launch_march_mask<G2Fam, march_key(CVS_G2_MASK_LINES, CVS_STEER_MAP), true>(g, a, tt, grid, stream, info, "g2_march<lines@map>");
-}
-
+CVS_FORM_F32(G2Fam, 8)
+CVS_FORM_F32(G2Fam, 9)
+CVS_FORM_F32(G2Fam, 10)
+CVS_FORM_F32(G2Fam, 11)
 }  // namespace cvs

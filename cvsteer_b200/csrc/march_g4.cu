@@ -1,27 +1,9 @@
-// G4/H4 instantiations of the marching kernel (reference cvsteer/SteerableFiltersG4.cpp:67-122 fused).
-#include "march_launch.cuh"
+// G4/H4 fused kernels with fp32 planes (reference cvsteer/SteerableFiltersG4.cpp:67-122 fused): the run-time-mask
+// kernel, the basis and steering at an angle map (march_launch.cuh's G4 table, entries 0-2).
+#include "march_forms.cuh"
 
 namespace cvs {
-
-// march_g4_steer.cu: steer mask at one scalar angle (G4.cpp:114-122) and at this library's G4 theta_d
-cudaError_t launch_march_g4_steer_other(const BatchGeom& g, const MarchArgs& a, const TapTable<G4Fam::NSETS, G4Fam::R>& tt, dim3 grid,
-                                        cudaStream_t stream, LaunchInfo* info);
-
-cudaError_t launch_march_g4(const FamilyTaps& taps, const BatchGeom& g, const MarchArgs& a, bool dom, cudaStream_t stream, LaunchInfo* info)
-{
-    (void)dom;
-    TapTable<G4Fam::NSETS, G4Fam::R> tt;
-    fill_tap_table<G4Fam>(taps, tt);
-    const int out_rows = g.out_row_end - g.out_row_begin;
-    const dim3 grid((g.cols + MARCH_TW - 1) / MARCH_TW, (out_rows + G4Fam::BH - 1) / G4Fam::BH, g.n);
-    static const bool dyn_only = getenv("CVS_G4_DYN_ONLY") != nullptr;  // A/B switch
-    if (a.mask == CVS_G4_MASK_STEER && !dyn_only) {
-        if (a.steer_source == CVS_STEER_MAP)
-            return launch_march_mask<G4Fam, march_key(CVS_G4_MASK_STEER, CVS_STEER_MAP), true>(g, a, tt, grid, stream, info, "g4_march<steer@map>");
-        return launch_march_g4_steer_other(g, a, tt, grid, stream, info);
-    }
-    if (a.mask == CVS_G4_MASK_BASIS) return launch_march_mask<G4Fam, CVS_G4_MASK_BASIS, true>(g, a, tt, grid, stream, info, "g4_march<basis>");
-    return launch_march_mask<G4Fam, 0u>(g, a, tt, grid, stream, info, "g4_march<dyn>");
-}
-
+CVS_FORM_F32(G4Fam, 0)
+CVS_FORM_F32(G4Fam, 1)
+CVS_FORM_F32(G4Fam, 2)
 }  // namespace cvs

@@ -1,7 +1,7 @@
-// G4 fused steer kernels at a scalar angle and at theta_d with bf16 output planes (see march_out16.cuh).
-#include "march_out16.cuh"
+// G4/H4 fused steering kernels at a scalar angle and at theta_d with bf16 planes from fp32 frames (G4 entries 3-4).
+#include "march_forms.cuh"
 
 namespace cvs {
-template cudaError_t launch_march_g4_out16_other<__nv_bfloat16>(const BatchGeom&, const MarchArgs&, const TapTable<G4Fam::NSETS, G4Fam::R>&, dim3, cudaStream_t,
-                                                      LaunchInfo*);
+CVS_FORM(G4Fam, 3, __nv_bfloat16, float)
+CVS_FORM(G4Fam, 4, __nv_bfloat16, float)
 }  // namespace cvs

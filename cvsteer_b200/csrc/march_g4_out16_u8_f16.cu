@@ -1,6 +1,8 @@
-// G4 fused basis and steer@map kernels with 8-bit input and f16 output planes (see march_out16.cuh).
-#include "march_out16.cuh"
+// G4/H4 fused basis and steer@map kernels with f16 planes from 8-bit frames (G4 entries 0-2).
+#include "march_forms.cuh"
 
 namespace cvs {
-template cudaError_t launch_march_g4_out16<__half, unsigned char>(const FamilyTaps&, const BatchGeom&, const MarchArgs&, cudaStream_t, LaunchInfo*);
+CVS_FORM(G4Fam, 0, __half, unsigned char)
+CVS_FORM(G4Fam, 1, __half, unsigned char)
+CVS_FORM(G4Fam, 2, __half, unsigned char)
 }  // namespace cvs

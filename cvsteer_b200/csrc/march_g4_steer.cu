@@ -1,15 +1,8 @@
-// G4/H4 marching kernel, steer mask (g4, h4, magnitude, phase) at ONE scalar angle (reference SteerableFiltersG4.cpp:114-122
-// fused with the basis stage) and at the in-kernel dominant angle (this library's G4 orientation analysis, CVS_G4_THETA).
-#include "march_launch.cuh"
+// G4/H4 fused kernels with fp32 planes: steering at one scalar angle (reference SteerableFiltersG4.cpp:114-122) and at
+// this library's G4 theta_d (entries 3-4).
+#include "march_forms.cuh"
 
 namespace cvs {
-
-cudaError_t launch_march_g4_steer_other(const BatchGeom& g, const MarchArgs& a, const TapTable<G4Fam::NSETS, G4Fam::R>& tt, dim3 grid,
-                                        cudaStream_t stream, LaunchInfo* info)
-{
-    if (a.steer_source == CVS_STEER_SCALAR)
-        return launch_march_mask<G4Fam, march_key(CVS_G4_MASK_STEER, CVS_STEER_SCALAR), true>(g, a, tt, grid, stream, info, "g4_march<steer@scalar>");
-    return launch_march_mask<G4Fam, march_key(CVS_G4_MASK_STEER, CVS_STEER_DOMINANT), true>(g, a, tt, grid, stream, info, "g4_march<steer@theta_d>");
-}
-
+CVS_FORM_F32(G4Fam, 3)
+CVS_FORM_F32(G4Fam, 4)
 }  // namespace cvs

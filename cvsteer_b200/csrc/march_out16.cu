@@ -1,69 +1,8 @@
-// 16-bit output planes: choice between the fused 16-bit kernels (march_out16.cuh) and the narrowing kernel the fallback
-// (capi.cu: fp32 kernel into scratch, then k_narrow) ends with.
-#include "march_out16.cuh"
+// 16-bit output planes without a fused 16-bit kernel (capi.cu: fp32 kernel into scratch, then k_narrow), and 8-bit frames
+// widened to fp32 for the host-buffer path.
+#include "march_launch.cuh"
 
 namespace cvs {
-
-// Two 16-bit pixels per thread are one 4-byte store per plane: planes, pitch and frame stride multiples of 4, even width (the
-// clamped last pair stays aligned); the fp32 angle pairs stay 8-byte loads (map pitch = 2 x out_pitch).
-static bool pair_store16_ok(const BatchGeom& g, const MarchArgs& a)
-{
-    if ((g.cols & 1) || (g.out_pitch & 3) || (g.out_frame_stride & 3)) return false;
-    for (int p = 0; p < MARCH_MAX_OUT; ++p)
-        if (a.out[p] && ((uintptr_t)a.out[p] & 3)) return false;
-    return !(a.steer_source == CVS_STEER_MAP && ((uintptr_t)a.theta_map & 7));
-}
-
-template <class Fam>
-static bool default_taps(const FamilyTaps& taps)
-{
-    TapTable<Fam::NSETS, Fam::R> tt;
-    fill_tap_table<Fam>(taps, tt);
-    return taps_are_baked<Fam>(tt);
-}
-
-cudaError_t launch_basis_fused16(int family, int fmt, const FamilyTaps& taps, const BatchGeom& g, unsigned mask, const SteerSpec& st,
-                                 void* const* outs, cudaStream_t stream, LaunchInfo* info, bool* taken)
-{
-    *taken = false;
-    if (fmt != 1 && fmt != 2) return cudaErrorInvalidValue;
-    // 8-bit frames take the fused kernels where the fp32-output launch would stage them by TMA (march_launch.cuh); the
-    // cooperative `ldg-u8` loader stays on the fallback
-    const int px = uses_march_path(family, taps.width) ? out16_kernel_px(family, mask, st.source, g.in_u8) : 0;
-    if (!px || !tma_eligible(g, family == 2 ? G2Fam::R : G4Fam::R)) return cudaSuccess;
-    if (!(family == 2 ? default_taps<G2Fam>(taps) : default_taps<G4Fam>(taps))) return cudaSuccess;
-    const int nplanes = family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES;
-    const MarchArgs a = make_args(g, mask, st, reinterpret_cast<float* const*>(outs), nplanes);
-    if (px == 2 && !pair_store16_ok(g, a)) return cudaSuccess;
-    if (g.out_row_end <= g.out_row_begin || g.cols <= 0 || g.n <= 0) return cudaErrorInvalidValue;
-    *taken = true;
-    // gridDim.z carries the frame index: batches beyond 65535 frames go out as several launches (as launch_basis_fused)
-    for (int f0 = 0; f0 < g.n; f0 += 65535) {
-        BatchGeom gc = g;
-        MarchArgs ac = a;
-        gc.n = g.n - f0 < 65535 ? g.n - f0 : 65535;
-        gc.in = static_cast<const char*>(g.in) + (size_t)f0 * g.in_frame_stride;
-        ac.in = gc.in;
-        for (int p = 0; p < MARCH_MAX_OUT; ++p)
-            if (ac.out[p]) ac.out[p] = reinterpret_cast<float*>(reinterpret_cast<char*>(a.out[p]) + (size_t)f0 * g.out_frame_stride);
-        if (ac.theta_map)  // 4-byte elements in the outputs' element layout
-            ac.theta_map = reinterpret_cast<const float*>(reinterpret_cast<const char*>(a.theta_map) + 2 * (size_t)f0 * g.out_frame_stride);
-        if (ac.pyr_out) ac.pyr_out = reinterpret_cast<float*>(reinterpret_cast<char*>(a.pyr_out) + (size_t)f0 * g.next_frame_stride);
-        cudaError_t e;
-        if (family == 2 && g.in_u8)
-            e = fmt == 1 ? launch_march_g2_out16<__half, unsigned char>(taps, gc, ac, stream, info)
-                         : launch_march_g2_out16<__nv_bfloat16, unsigned char>(taps, gc, ac, stream, info);
-        else if (family == 2)
-            e = fmt == 1 ? launch_march_g2_out16<__half>(taps, gc, ac, stream, info) : launch_march_g2_out16<__nv_bfloat16>(taps, gc, ac, stream, info);
-        else if (g.in_u8)
-            e = fmt == 1 ? launch_march_g4_out16<__half, unsigned char>(taps, gc, ac, stream, info)
-                         : launch_march_g4_out16<__nv_bfloat16, unsigned char>(taps, gc, ac, stream, info);
-        else
-            e = fmt == 1 ? launch_march_g4_out16<__half>(taps, gc, ac, stream, info) : launch_march_g4_out16<__nv_bfloat16>(taps, gc, ac, stream, info);
-        if (e != cudaSuccess) return e;
-    }
-    return cudaSuccess;
-}
 
 struct NarrowArgs {
     const float* src[MARCH_MAX_OUT];

@@ -30,11 +30,11 @@ DOM, SCALAR, MAP = capi.STEER_DOMINANT, capi.STEER_SCALAR, capi.STEER_MAP
 SCALARS = (1.5707, 1.5709, -1.5707, -1.5709, 0.7)
 
 # --------------------------------------------------------------------------------------------------------------------------
-# The kernel forms (march_launch.cuh launch_march_mask and the launch_march_g2 / launch_march_g4 dispatch):
+# The kernel forms (the table of forms and launch_form in march_launch.cuh / march_forms.cuh):
 #   every static mask: /tma/imm-taps (default taps, TMA-eligible fp32), /tma (other taps at the default width), /ldg (an
 #   fp32 frame the TMA cannot address), /tma-u8 and /ldg-u8 (8-bit frames);
-#   /tma/imm-taps/2px where the mask has a two-pixel instantiation (CVS_MARCH_PX2 = 1: M2, lines, steer5, M2 and lines at
-#   a scalar, M2 at a map) and the output layout allows pair stores (even width);
+#   /tma/imm-taps/2px where the mask has a two-pixel instantiation (M2, lines, steer5, M2 and lines at a scalar, M2 at a
+#   map) and the output layout allows pair stores (even width);
 #   the run-time-mask kernels (<dyn>) have no baked-tap form;
 #   widths other than the family default take the two-kernel generic path (generic_w<width>).
 # --------------------------------------------------------------------------------------------------------------------------

@@ -1,5 +1,6 @@
 #!/bin/bash
 # Alternating A/B of the shipped library against tuning variants: ROUNDS x (base, each variant), kernel-table rows matching $ONLY
+# Build variant <v> from cvsteer_b200/csrc with: make OBJDIR=build/var_<v> OUT=../variants/libcvsteer_b200_<v>.so EXTRA="-D..."
 ONLY=${ONLY:-M2}; SIZES=${SIZES:-1080p,4k}; ROUNDS=${ROUNDS:-3}; ITERS=${ITERS:-100}
 for i in $(seq $ROUNDS); do for v in base $VARIANTS; do
   if [ $v = base ]; then unset CVS_LIB; else export CVS_LIB=$PWD/cvsteer_b200/variants/libcvsteer_b200_$v.so; fi

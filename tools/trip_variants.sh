@@ -1,5 +1,6 @@
 #!/bin/bash
 # A/B of tuning variants (cvsteer_b200/variants/*.so): kernel table rows selected by $ONLY for the shipped library and each variant
+# Build variant <v> from cvsteer_b200/csrc with: make OBJDIR=build/var_<v> OUT=../variants/libcvsteer_b200_<v>.so EXTRA="-D..."
 mkdir -p gpurun_out
 ONLY=${ONLY:-g4}
 SIZES=${SIZES:-4k}
