@@ -81,23 +81,24 @@ def _host_frames(x: torch.Tensor):
     return x.dtype == torch.uint8, x.stride(1) * es, x.stride(0) * es
 
 
-def _bank_angles(thetas, mask: int):
-    """float array of the bank's angles; the angle count and the mask checked before anything touches a device."""
+def _bank_angles(thetas, mask: int, bank_planes: int):
+    """float array of the bank's angles; the angle count and the mask (bits of the family's bank planes) checked before
+    anything touches a device."""
     th = [float(t) for t in thetas]
     if not 1 <= len(th) <= capi.BANK_MAX_ANGLES:
         raise capi.CvsError(capi.ERR_INVALID_ARG, f"a bank steers to 1..{capi.BANK_MAX_ANGLES} angles, got {len(th)}")
-    if not mask or mask & ~capi.G2_BANK_PLANES:
-        raise capi.CvsError(capi.ERR_INVALID_ARG, f"bank mask 0x{mask:x}: bank planes are 0x{capi.G2_BANK_PLANES:x}")
+    if not mask or mask & ~bank_planes:
+        raise capi.CvsError(capi.ERR_INVALID_ARG, f"bank mask 0x{mask:x}: bank planes are 0x{bank_planes:x}")
     return (C.c_float * len(th))(*th)
 
 
-def _bank_layout(outs: Dict[int, torch.Tensor], planes, shape_angle, shape_once):
-    """(out_pitch, out_frame_stride, angle_stride) in bytes shared by the bank's planes: per-angle planes are
-    [N, n, rows, cols] views, theta / strength [n, rows, cols]; any strides with unit column stride."""
+def _bank_layout(outs: Dict[int, torch.Tensor], planes, shape_angle, shape_once, per_angle_mask: int):
+    """(out_pitch, out_frame_stride, angle_stride) in bytes shared by the bank's planes: per-angle planes (bits of
+    per_angle_mask) are [N, n, rows, cols] views, G2's theta / strength [n, rows, cols]; any strides with unit column stride."""
     lay = set()
     for p in planes:
         t = outs[p]
-        per_angle = capi.G2_MASK_STEER5 >> p & 1
+        per_angle = per_angle_mask >> p & 1
         want = shape_angle if per_angle else shape_once
         if tuple(t.shape) != want or t.stride(-1) != 1:
             raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"output plane {p}: need {want} with unit column stride, got {tuple(t.shape)}")
@@ -121,6 +122,8 @@ def _stream_ptr(stream):
 class _FusedBatch:
     _prefix = ""
     _names: Sequence[str] = ()
+    _bank_planes = 0      # mask bits a steering bank takes
+    _bank_per_angle = 0   # ... those of them written once per angle
 
     def __init__(self, width: int, spacing: float, device: Optional[int] = None):
         self._lib = capi.lib()
@@ -207,6 +210,74 @@ class _FusedBatch:
                 cur = nxt if fuse else pyr_down(cur, stream=kw.get("stream"))
         return res
 
+    def steer_bank(self, frames: torch.Tensor, thetas, mask: Optional[int] = None, outs: Optional[Dict[int, torch.Tensor]] = None,
+                   out_dtype: torch.dtype = torch.float32, band: Optional[Band] = None, next_level: Optional[torch.Tensor] = None,
+                   stream=None) -> Dict[str, torch.Tensor]:
+        """Steering bank (cvs_g2_steer_bank_dev / cvs_g4_steer_bank_dev): one filtering pass, then the planes of `mask` (default:
+        every per-angle plane of the family) at every angle of `thetas` (1..16 of them).  Returns {name: tensor}:
+        [N, n, out_rows, cols] for the per-angle planes (G2: g2, h2, e, magnitude, phase; G4: g4, h4, magnitude, phase),
+        [n, out_rows, cols] for G2's theta and strength.  Each per-angle plane k is, bit for bit, that plane of
+        run(frames, G2_MASK_STEER5 / G4_MASK_STEER, STEER_SCALAR, thetas[k]) -- for G4 on uint8 frames, of that call on
+        frames.float() -- and G2's theta / strength those of run(frames, G2_MASK_ORIENT).
+        outs: optional {plane: tensor} of those shapes with any strides of unit column stride, e.g. a [n, N, rows, cols]
+        tensor seen through .transpose(0, 1); the planes share one row pitch and frame stride.  band and next_level as in run()."""
+        mask = self._bank_per_angle if mask is None else mask
+        th = _bank_angles(thetas, mask, self._bank_planes)
+        x = _as_batch(frames)
+        if x.device.index != self.device:
+            raise capi.CvsError(capi.ERR_INVALID_ARG, f"frames live on cuda:{x.device.index}, this handle on cuda:{self.device}")
+        n, rows, cols = x.shape
+        out_rows = rows if band is None else band.row_end - band.row_begin
+        nplanes = len(self._names)
+        planes = [p for p in range(nplanes) if mask >> p & 1]
+        fmt = _out_format(out_dtype)
+        shape_angle, shape_once = (len(th), n, out_rows, cols), (n, out_rows, cols)
+        if outs is None:
+            outs = {p: torch.empty(shape_angle if self._bank_per_angle >> p & 1 else shape_once, dtype=out_dtype, device=x.device)
+                    for p in planes}
+        for p in planes:
+            if p not in outs:
+                raise capi.CvsError(capi.ERR_INVALID_ARG, f"no output plane for {p}")
+            if outs[p].dtype != out_dtype or outs[p].device != x.device:
+                raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"output plane {p}: need {out_dtype} on {x.device}")
+        pitch, fstride, astride = _bank_layout(outs, planes, shape_angle, shape_once, self._bank_per_angle)
+        arr = (C.c_void_p * nplanes)()
+        for p in planes:
+            arr[p] = outs[p].data_ptr()
+        b = _batch_struct(x, pitch, fstride, band)
+        if next_level is not None:
+            want = (n, (rows + 1) // 2, (cols + 1) // 2)
+            if tuple(next_level.shape) != want or next_level.dtype != torch.float32 or not next_level.is_contiguous():
+                raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"next_level must be contiguous float32 {want}")
+            b.next_level = next_level.data_ptr()
+            b.next_pitch, b.next_frame_stride = want[2] * 4, want[1] * want[2] * 4
+        with torch.cuda.device(self.device):
+            fn = getattr(self._lib, f"cvs_{self._prefix}_steer_bank_dev")
+            capi.check(fn(self._h, C.byref(b), th, len(th), mask, arr, astride, _stream_ptr(stream), fmt))
+        return {self._names[p]: outs[p] for p in planes}
+
+    def steer_bank_host(self, frames_host: torch.Tensor, thetas, mask: int, outs_host: Dict[int, torch.Tensor]):
+        """Host-buffer twin of steer_bank (cvs_g2_steer_bank_host / cvs_g4_steer_bank_host): pinned float32 or uint8 frames
+        [n, rows, cols] in, pinned planes out ([N, n, rows, cols] per angle, [n, rows, cols] for G2's theta / strength, one
+        dtype that selects the format)."""
+        th = _bank_angles(thetas, mask, self._bank_planes)
+        x = frames_host
+        u8, step, fstride = _host_frames(x)
+        n, rows, cols = x.shape
+        fmt, _ = _host_format(outs_host)
+        nplanes = len(self._names)
+        planes = [p for p in range(nplanes) if mask >> p & 1]
+        missing = [p for p in planes if p not in outs_host]
+        if missing:
+            raise capi.CvsError(capi.ERR_INVALID_ARG, f"no output plane for {missing}")
+        pitch, ofs, astride = _bank_layout(outs_host, planes, (len(th), n, rows, cols), (n, rows, cols), self._bank_per_angle)
+        arr = (C.c_void_p * nplanes)()
+        for p in planes:
+            arr[p] = outs_host[p].data_ptr()
+        fn = getattr(self._lib, f"cvs_{self._prefix}_steer_bank_host")
+        capi.check(fn(self._h, C.c_void_p(x.data_ptr()), int(u8), n, rows, cols, step, fstride, th, len(th), mask, arr, pitch, ofs, astride,
+                      fmt))
+
     def last_launch(self):
         g = (C.c_int * 3)()
         blk, sm = C.c_int(), C.c_int()
@@ -218,6 +289,8 @@ class _FusedBatch:
 class G2Batch(_FusedBatch):
     _prefix = "g2"
     _names = capi.G2_PLANE_NAMES
+    _bank_planes = capi.G2_BANK_PLANES
+    _bank_per_angle = capi.G2_MASK_STEER5
 
     def __init__(self, width: int = 4, spacing: float = 0.67, device: Optional[int] = None):
         super().__init__(width, spacing, device)
@@ -244,70 +317,11 @@ class G2Batch(_FusedBatch):
             capi.check(self._lib.cvs_g2_run_batch_host_fmt(*args, fmt))
 
 
-    def steer_bank(self, frames: torch.Tensor, thetas, mask: int = capi.G2_MASK_STEER5, outs: Optional[Dict[int, torch.Tensor]] = None,
-                   out_dtype: torch.dtype = torch.float32, band: Optional[Band] = None, next_level: Optional[torch.Tensor] = None,
-                   stream=None) -> Dict[str, torch.Tensor]:
-        """Steering bank (cvs_g2_steer_bank_dev): one filtering pass, then the planes of `mask` at every angle of `thetas`
-        (1..16 of them).  Returns {name: tensor}: [N, n, out_rows, cols] for the per-angle planes (g2, h2, e, magnitude,
-        phase), [n, out_rows, cols] for theta and strength.  Each per-angle plane k is, bit for bit, that plane of
-        run(frames, G2_MASK_STEER5, STEER_SCALAR, thetas[k]); theta / strength those of run(frames, G2_MASK_ORIENT).
-        outs: optional {plane: tensor} of those shapes with any strides of unit column stride, e.g. a [n, N, rows, cols]
-        tensor seen through .transpose(0, 1); the planes share one row pitch and frame stride.  band and next_level as in run()."""
-        th = _bank_angles(thetas, mask)
-        x = _as_batch(frames)
-        if x.device.index != self.device:
-            raise capi.CvsError(capi.ERR_INVALID_ARG, f"frames live on cuda:{x.device.index}, this handle on cuda:{self.device}")
-        n, rows, cols = x.shape
-        out_rows = rows if band is None else band.row_end - band.row_begin
-        planes = [p for p in range(capi.G2_NPLANES) if mask >> p & 1]
-        fmt = _out_format(out_dtype)
-        shape_angle, shape_once = (len(th), n, out_rows, cols), (n, out_rows, cols)
-        if outs is None:
-            outs = {p: torch.empty(shape_angle if capi.G2_MASK_STEER5 >> p & 1 else shape_once, dtype=out_dtype, device=x.device)
-                    for p in planes}
-        for p in planes:
-            if p not in outs:
-                raise capi.CvsError(capi.ERR_INVALID_ARG, f"no output plane for {p}")
-            if outs[p].dtype != out_dtype or outs[p].device != x.device:
-                raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"output plane {p}: need {out_dtype} on {x.device}")
-        pitch, fstride, astride = _bank_layout(outs, planes, shape_angle, shape_once)
-        arr = (C.c_void_p * capi.G2_NPLANES)()
-        for p in planes:
-            arr[p] = outs[p].data_ptr()
-        b = _batch_struct(x, pitch, fstride, band)
-        if next_level is not None:
-            want = (n, (rows + 1) // 2, (cols + 1) // 2)
-            if tuple(next_level.shape) != want or next_level.dtype != torch.float32 or not next_level.is_contiguous():
-                raise capi.CvsError(capi.ERR_SIZE_MISMATCH, f"next_level must be contiguous float32 {want}")
-            b.next_level = next_level.data_ptr()
-            b.next_pitch, b.next_frame_stride = want[2] * 4, want[1] * want[2] * 4
-        with torch.cuda.device(self.device):
-            capi.check(self._lib.cvs_g2_steer_bank_dev(self._h, C.byref(b), th, len(th), mask, arr, astride, _stream_ptr(stream), fmt))
-        return {self._names[p]: outs[p] for p in planes}
-
-    def steer_bank_host(self, frames_host: torch.Tensor, thetas, mask: int, outs_host: Dict[int, torch.Tensor]):
-        """Host-buffer twin of steer_bank (cvs_g2_steer_bank_host): pinned float32 or uint8 frames [n, rows, cols] in, pinned
-        planes out ([N, n, rows, cols] per angle, [n, rows, cols] for theta / strength, one dtype that selects the format)."""
-        th = _bank_angles(thetas, mask)
-        x = frames_host
-        u8, step, fstride = _host_frames(x)
-        n, rows, cols = x.shape
-        fmt, _ = _host_format(outs_host)
-        planes = [p for p in range(capi.G2_NPLANES) if mask >> p & 1]
-        missing = [p for p in planes if p not in outs_host]
-        if missing:
-            raise capi.CvsError(capi.ERR_INVALID_ARG, f"no output plane for {missing}")
-        pitch, ofs, astride = _bank_layout(outs_host, planes, (len(th), n, rows, cols), (n, rows, cols))
-        arr = (C.c_void_p * capi.G2_NPLANES)()
-        for p in planes:
-            arr[p] = outs_host[p].data_ptr()
-        capi.check(self._lib.cvs_g2_steer_bank_host(self._h, C.c_void_p(x.data_ptr()), int(u8), n, rows, cols, step, fstride, th, len(th),
-                                                    mask, arr, pitch, ofs, astride, fmt))
-
-
 class G4Batch(_FusedBatch):
     _prefix = "g4"
     _names = capi.G4_PLANE_NAMES
+    _bank_planes = capi.G4_BANK_PLANES
+    _bank_per_angle = capi.G4_MASK_STEER
 
     def __init__(self, width: int = 6, spacing: float = 0.5, device: Optional[int] = None):
         super().__init__(width, spacing, device)

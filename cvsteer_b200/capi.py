@@ -37,6 +37,7 @@ G2_MASK_STEER5 = bit(G2T) | bit(H2T) | bit(E) | bit(MAG) | bit(PHASE)
 G4_MASK_BASIS = 0x000007FF
 G4_MASK_STEER = bit(G4T) | bit(H4T) | bit(MAG4) | bit(PHASE4)
 G2_BANK_PLANES = G2_MASK_STEER5 | bit(THETA) | bit(STRENGTH)  # per angle: the STEER5 planes; once per pixel: theta, strength
+G4_BANK_PLANES = G4_MASK_STEER  # per angle: g4, h4, magnitude, phase (no theta_d / strength: include/cvsteer_c.h)
 BANK_MAX_ANGLES = 16
 STEER_DOMINANT, STEER_SCALAR, STEER_MAP = 0, 1, 2
 OUT_F32, OUT_F16, OUT_BF16 = 0, 1, 2
@@ -121,6 +122,10 @@ _SIGS = {
     "cvs_g2_steer_bank_dev": (C.c_int, [C.c_void_p, C.POINTER(Batch), _fp, C.c_int, C.c_uint, C.POINTER(C.c_void_p), C.c_size_t,
                                         C.c_void_p, C.c_int]),
     "cvs_g2_steer_bank_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, _fp,
+                                         C.c_int, C.c_uint, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t, C.c_size_t, C.c_int]),
+    "cvs_g4_steer_bank_dev": (C.c_int, [C.c_void_p, C.POINTER(Batch), _fp, C.c_int, C.c_uint, C.POINTER(C.c_void_p), C.c_size_t,
+                                        C.c_void_p, C.c_int]),
+    "cvs_g4_steer_bank_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, _fp,
                                          C.c_int, C.c_uint, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t, C.c_size_t, C.c_int]),
     "cvs_to_u8_dev": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_size_t, C.c_float, C.c_void_p,
                                 C.c_size_t, C.c_size_t, C.c_void_p]),

@@ -336,19 +336,24 @@ int run_fused_fmt(Filter* f, const BatchGeom& g, unsigned mask, const SteerSpec&
     return CVS_OK;
 }
 
-// Steering bank (cvs_g2_steer_bank_dev): the fused bank kernel when its forms apply, otherwise the calls the contract names --
-// one STEER5 launch per scalar angle and one ORIENT launch at theta_d when theta_d or strength is wanted -- with the planes they
-// write but the caller did not select in stream-ordered scratch of the caller's layout.  Both give the same bits.
+// Steering bank (cvs_g2_steer_bank_dev / cvs_g4_steer_bank_dev): the family's fused bank kernel when its forms apply, otherwise
+// the calls the contract names, with the planes they write but the caller did not select in stream-ordered scratch of the
+// caller's layout.  Both give the same bits.
+//   G2: one STEER5 launch per scalar angle and one ORIENT launch at theta_d when theta_d or strength is wanted.
+//   G4: one STEER launch per scalar angle, on the frames widened to fp32 when they are 8-bit (the contract's reference: the
+//       8-bit single-angle kernels with fp32 planes do not prescale their taps, see run_batch_host's `widen`).
 int run_bank(Filter* f, const BatchGeom& g, const BankSpec& bk, int fmt, cudaStream_t stream, int slot = 0, int nslots = 1)
 {
     CU_TRY(cudaSetDevice(f->device));
+    const bool g4 = f->family == 4;
     bool taken = false;
-    CU_TRY(launch_g2_bank(fmt, f->taps, g, bk, stream, &f->last, &taken));
+    CU_TRY((g4 ? launch_g4_bank : launch_g2_bank)(fmt, f->taps, g, bk, stream, &f->last, &taken));
     if (taken) return CVS_OK;
-    const unsigned orient_bits = CVS_BIT(CVS_THETA) | CVS_BIT(CVS_STRENGTH);
-    const bool steer = (bk.mask & CVS_G2_MASK_STEER5) != 0, orient = (bk.mask & orient_bits) != 0;
-    unsigned scr = 0;  // planes written to scratch: E of the ORIENT launch always (the caller's E planes hold E(theta_k))
-    if (steer) scr |= CVS_G2_MASK_STEER5 & ~bk.mask;
+    const unsigned per_angle = g4 ? (unsigned)CVS_G4_MASK_STEER : (unsigned)CVS_G2_MASK_STEER5;
+    const unsigned orient_bits = g4 ? 0u : CVS_BIT(CVS_THETA) | CVS_BIT(CVS_STRENGTH);
+    const bool steer = (bk.mask & per_angle) != 0, orient = (bk.mask & orient_bits) != 0;
+    unsigned scr = 0;  // planes written to scratch: G2's E of the ORIENT launch always (the caller's E planes hold E(theta_k))
+    if (steer) scr |= per_angle & ~bk.mask;
     if (orient) scr |= CVS_G2_MASK_ORIENT & ~(bk.mask & orient_bits);
     const size_t set_bytes = (size_t)(g.n - 1) * g.out_frame_stride + (size_t)(g.out_row_end - g.out_row_begin) * g.out_pitch;
     void* scratch = nullptr;
@@ -360,15 +365,27 @@ int run_bank(Filter* f, const BatchGeom& g, const BankSpec& bk, int fmt, cudaStr
     char first[sizeof(f->last.name)] = "";
     BatchGeom gk = g;
     int rc = CVS_OK;
+    void* wide = nullptr;  // G4, 8-bit frames: the buffer rows widened to dense fp32 frames (the layout of x.float())
+    if (g4 && g.in_u8) {
+        const size_t wpitch = (size_t)g.cols * 4, wfs = wpitch * (size_t)g.buf_rows;
+        if (cudaError_t e = cudaMallocAsync(&wide, wfs * (size_t)g.n, stream); e != cudaSuccess) {
+            if (scr) cudaFreeAsync(scratch, stream);
+            CU_TRY(e);
+        }
+        const cudaError_t e = launch_widen(static_cast<const unsigned char*>(g.in), g.in_pitch, g.in_frame_stride, static_cast<float*>(wide), wpitch,
+                                           wfs, g.n, g.buf_rows, g.cols, stream);
+        if (e != cudaSuccess) rc = fail(CVS_ERR_CUDA, "widen: %s", cudaGetErrorString(e));
+        gk.in = wide, gk.in_u8 = false, gk.in_pitch = wpitch, gk.in_frame_stride = wfs;
+    }
     for (int k = 0; steer && k < bk.n_angles && rc == CVS_OK; ++k) {
         void* outs[CVS_G2_NPLANES] = {nullptr};
         for (int q = 0; q < CVS_G2_NPLANES; ++q)
-            if (CVS_G2_MASK_STEER5 >> q & 1u) outs[q] = pick(q, (size_t)k * bk.angle_stride);
+            if (per_angle >> q & 1u) outs[q] = pick(q, (size_t)k * bk.angle_stride);
         SteerSpec st{};
         st.source = CVS_STEER_SCALAR;
         st.cos_t = bk.cos_t[k];
         st.sin_t = bk.sin_t[k];
-        rc = run_fused_fmt(f, gk, CVS_G2_MASK_STEER5, st, outs, fmt, stream, slot, nslots);
+        rc = run_fused_fmt(f, gk, per_angle, st, outs, fmt, stream, slot, nslots);
         if (!first[0]) snprintf(first, sizeof(first), "%s", f->last.name);
         gk.next_level = nullptr;  // the first launch emitted it
     }
@@ -380,8 +397,10 @@ int run_bank(Filter* f, const BatchGeom& g, const BankSpec& bk, int fmt, cudaStr
         rc = run_fused_fmt(f, gk, CVS_G2_MASK_ORIENT, st, outs, fmt, stream, slot, nslots);
         if (!first[0]) snprintf(first, sizeof(first), "%s", f->last.name);
     }
+    const cudaError_t ew = wide ? cudaFreeAsync(wide, stream) : cudaSuccess;
     const cudaError_t e = scr ? cudaFreeAsync(scratch, stream) : cudaSuccess;
     if (rc != CVS_OK) return rc;
+    CU_TRY(ew);
     CU_TRY(e);
     snprintf(f->last.name, sizeof(f->last.name), "bank-fallback:%s", first);
     return CVS_OK;
@@ -762,17 +781,21 @@ extern "C" int cvs_g4_run_batch_dev_fmt(cvs_g4* h, const cvs_batch* b, unsigned 
 }
 
 // Steering-bank arguments, checked before the handle is looked at and before any CUDA call.  out_rows: rows of one output plane.
-static int check_bank(const float* thetas, int n_angles, unsigned mask, void* const* outs, int fmt, int cols, int n, int out_rows, size_t out_pitch,
-                      size_t out_frame_stride, size_t angle_stride)
+// family: 2 or 4 -- its bank planes, the per-angle ones among them and its plane count.
+static int check_bank(int family, const float* thetas, int n_angles, unsigned mask, void* const* outs, int fmt, int cols, int n, int out_rows,
+                      size_t out_pitch, size_t out_frame_stride, size_t angle_stride)
 {
+    const unsigned planes = family == 2 ? (unsigned)CVS_G2_BANK_PLANES : (unsigned)CVS_G4_BANK_PLANES;
+    const unsigned per_angle = family == 2 ? (unsigned)CVS_G2_MASK_STEER5 : (unsigned)CVS_G4_MASK_STEER;
+    const int nplanes = family == 2 ? (int)CVS_G2_NPLANES : (int)CVS_G4_NPLANES;
     if (n_angles < 1 || n_angles > CVS_BANK_MAX_ANGLES) return fail(CVS_ERR_INVALID_ARG, "n_angles %d outside [1, %d]", n_angles, CVS_BANK_MAX_ANGLES);
     if (!thetas) return fail(CVS_ERR_INVALID_ARG, "thetas is null");
-    if (!mask || (mask & ~(unsigned)CVS_G2_BANK_PLANES)) return fail(CVS_ERR_INVALID_ARG, "mask 0x%x: bank planes are 0x%x", mask, (unsigned)CVS_G2_BANK_PLANES);
+    if (!mask || (mask & ~planes)) return fail(CVS_ERR_INVALID_ARG, "mask 0x%x: bank planes are 0x%x", mask, planes);
     if (!outs) return fail(CVS_ERR_INVALID_ARG, "outs is null");
-    for (int p = 0; p < CVS_G2_NPLANES; ++p)
+    for (int p = 0; p < nplanes; ++p)
         if ((mask >> p & 1u) && !outs[p]) return fail(CVS_ERR_INVALID_ARG, "outs[%d] is null but selected by mask", p);
     if (fmt != CVS_OUT_F32)
-        if (int rc = check_out16(fmt, cols, out_pitch, mask, CVS_G2_NPLANES, outs)) return rc;
+        if (int rc = check_out16(fmt, cols, out_pitch, mask, nplanes, outs)) return rc;
     const size_t esz = fmt == CVS_OUT_F32 ? 4 : 2;
     if (out_pitch < (size_t)cols * esz) return fail(CVS_ERR_INVALID_ARG, "out_pitch %zu < cols*%zu", out_pitch, esz);
     if ((out_frame_stride | angle_stride) & (esz - 1))
@@ -780,7 +803,7 @@ static int check_bank(const float* thetas, int n_angles, unsigned mask, void* co
     // no two (angle, frame) planes of one quantity overlap: sort the strides of the dimensions that have more than one plane
     struct Dim { long long count; size_t stride; } d[2];
     int nd = 0;
-    if ((mask & CVS_G2_MASK_STEER5) && n_angles > 1) d[nd++] = {n_angles, angle_stride};
+    if ((mask & per_angle) && n_angles > 1) d[nd++] = {n_angles, angle_stride};
     if (n > 1) d[nd++] = {n, out_frame_stride};
     if (nd == 2 && d[1].stride < d[0].stride) std::swap(d[0], d[1]);
     const size_t extent = (size_t)std::max(out_rows, 0) * out_pitch;
@@ -801,21 +824,32 @@ static BankSpec make_bank(const float* thetas, int n_angles, unsigned mask, void
     return bk;
 }
 
-extern "C" int cvs_g2_steer_bank_dev(cvs_g2* h, const cvs_batch* b, const float* thetas, int n_angles, unsigned mask, void* const* outs,
-                                     size_t angle_stride, void* stream, int out_format)
+static int steer_bank_dev(int family, Filter* f, const cvs_batch* b, const float* thetas, int n_angles, unsigned mask, void* const* outs,
+                          size_t angle_stride, void* stream, int out_format)
 {
     if (!b) return fail(CVS_ERR_INVALID_ARG, "batch is null");
     const int out_rows = b->full_rows > 0 ? b->out_row_end - b->out_row_begin : b->rows;
-    if (int rc = check_bank(thetas, n_angles, mask, outs, out_format, b->cols, b->n, out_rows, b->out_pitch, b->out_frame_stride, angle_stride))
+    if (int rc = check_bank(family, thetas, n_angles, mask, outs, out_format, b->cols, b->n, out_rows, b->out_pitch, b->out_frame_stride,
+                            angle_stride))
         return rc;
-    Filter* f = reinterpret_cast<Filter*>(h);
-    if (!f || f->family != 2) return fail(CVS_ERR_INVALID_ARG, "handle is null or not a G2 handle");
+    if (!f || f->family != family) return fail(CVS_ERR_INVALID_ARG, "handle is null or not a G%d handle", family);
     BatchGeom g;
     int rc = geom_from_batch(b, &g, out_format == CVS_OUT_F32 ? 4 : 2);
     if (rc) return rc;
     rc = check_band(g, f->taps.width, g.full_rows);
     if (rc) return rc;
     return run_bank(f, g, make_bank(thetas, n_angles, mask, outs, angle_stride), out_format, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int cvs_g2_steer_bank_dev(cvs_g2* h, const cvs_batch* b, const float* thetas, int n_angles, unsigned mask, void* const* outs,
+                                     size_t angle_stride, void* stream, int out_format)
+{
+    return steer_bank_dev(2, reinterpret_cast<Filter*>(h), b, thetas, n_angles, mask, outs, angle_stride, stream, out_format);
+}
+extern "C" int cvs_g4_steer_bank_dev(cvs_g4* h, const cvs_batch* b, const float* thetas, int n_angles, unsigned mask, void* const* outs,
+                                     size_t angle_stride, void* stream, int out_format)
+{
+    return steer_bank_dev(4, reinterpret_cast<Filter*>(h), b, thetas, n_angles, mask, outs, angle_stride, stream, out_format);
 }
 
 extern "C" int cvs_pyr_down_dev(int device, const cvs_batch* b, float* out, void* stream)
@@ -850,7 +884,7 @@ int check_in_u8(const void* in, int cols, size_t in_step)
 
 // in_u8: 8-bit frames (in_step / in_frame_stride in bytes of them), else fp32; the device holds them in the same element type.
 // fmt: cvs_out_format of the host output planes (out_step / out_frame_stride in bytes of them)
-// bank: a steering bank (G2) instead of one launch of `mask` -- its mask and host planes are `mask` / `outs`, per-angle plane p of
+// bank: a steering bank instead of one launch of `mask` -- its mask and host planes are `mask` / `outs`, per-angle plane p of
 // angle k at outs[p] + k * bank->angle_stride; each (plane, angle) pair is one more device plane per chunk and one more download
 int run_batch_host(Filter* f, int family, const void* in, bool in_u8, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
                    unsigned mask, int steer_source, float theta, void* const* outs, size_t out_step, size_t out_frame_stride, int fmt = CVS_OUT_F32,
@@ -872,7 +906,8 @@ int run_batch_host(Filter* f, int family, const void* in, bool in_u8, int n, int
     if (out_step < (size_t)cols * esz) return fail(CVS_ERR_INVALID_ARG, "step < cols*%zu", esz);
     if (!mask || (mask >> NPLANES)) return fail(CVS_ERR_INVALID_ARG, "mask 0x%x", mask);
     // device planes per frame: one per selected plane, or one per angle for a bank's per-angle planes
-    auto copies = [&](int p) { return bank && (CVS_G2_MASK_STEER5 >> p & 1u) ? bank->n_angles : 1; };
+    const unsigned per_angle = family == 2 ? (unsigned)CVS_G2_MASK_STEER5 : (unsigned)CVS_G4_MASK_STEER;
+    auto copies = [&](int p) { return bank && (per_angle >> p & 1u) ? bank->n_angles : 1; };
     int nout = 0;
     for (int p = 0; p < NPLANES; ++p)
         if (mask >> p & 1u) {
@@ -885,8 +920,9 @@ int run_batch_host(Filter* f, int family, const void* in, bool in_u8, int n, int
     // G4 steering at a scalar angle into fp32 planes: with the default taps the fp32-frame launch folds the steering factors
     // into the baked column taps (G4Fam::prescaled), which the fp32-output 8-bit kernel does not, so the two differ in the
     // last bits.  There the 8-bit chunk is widened on the device and runs the fp32-frame launch, which keeps the contract
-    // (the planes of the widened frames).  Every 16-bit format has fused 8-bit kernels with the same taps as the fp32 ones.
-    const bool widen = in_u8 && fmt == CVS_OUT_F32 && family == 4 && steer_source == CVS_STEER_SCALAR;
+    // (the planes of the widened frames).  Every 16-bit format has fused 8-bit kernels with the same taps as the fp32 ones.  A G4
+    // bank keeps the contract on 8-bit frames itself (run_bank), so its chunks stay 8-bit.
+    const bool widen = in_u8 && fmt == CVS_OUT_F32 && family == 4 && steer_source == CVS_STEER_SCALAR && !bank;
     const size_t wpitch = align_up((size_t)cols * 4, 128), wbytes = widen ? wpitch * rows : 0;  // fp32 frames; widened ones
     // chunk so that >= 4 chunks exist (pipeline depth) but each is large enough to amortise launch + copy latency: 64 MB of
     // fp32 frames.  8-bit frames count as the fp32 frames they stand for, so 1-byte input does not make chunks four times
@@ -1018,17 +1054,32 @@ extern "C" int cvs_g4_run_batch_host_u8(cvs_g4* h, const uint8_t* in, int n, int
                           out_step, out_frame_stride, out_format);
 }
 
-extern "C" int cvs_g2_steer_bank_host(cvs_g2* h, const void* in, int in_is_u8, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
-                                      const float* thetas, int n_angles, unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride,
-                                      size_t angle_stride, int out_format)
+static int steer_bank_host(int family, Filter* f, const void* in, int in_is_u8, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                           const float* thetas, int n_angles, unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride,
+                           size_t angle_stride, int out_format)
 {
-    if (int rc = check_bank(thetas, n_angles, mask, outs, out_format, cols, n, rows, out_step, out_frame_stride, angle_stride)) return rc;
+    if (int rc = check_bank(family, thetas, n_angles, mask, outs, out_format, cols, n, rows, out_step, out_frame_stride, angle_stride)) return rc;
     if (!in) return fail(CVS_ERR_INVALID_ARG, "in is null");
     const size_t in_esz = in_is_u8 ? 1 : 4;
     if (in_step < (size_t)cols * in_esz) return fail(CVS_ERR_INVALID_ARG, "in_step %zu < cols*%zu", in_step, in_esz);
     const BankSpec bk = make_bank(thetas, n_angles, mask, outs, angle_stride);
-    return run_batch_host(reinterpret_cast<Filter*>(h), 2, in, in_is_u8 != 0, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_SCALAR, 0.f, outs,
-                          out_step, out_frame_stride, out_format, &bk);
+    return run_batch_host(f, family, in, in_is_u8 != 0, n, rows, cols, in_step, in_frame_stride, mask, CVS_STEER_SCALAR, 0.f, outs, out_step,
+                          out_frame_stride, out_format, &bk);
+}
+
+extern "C" int cvs_g2_steer_bank_host(cvs_g2* h, const void* in, int in_is_u8, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                      const float* thetas, int n_angles, unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride,
+                                      size_t angle_stride, int out_format)
+{
+    return steer_bank_host(2, reinterpret_cast<Filter*>(h), in, in_is_u8, n, rows, cols, in_step, in_frame_stride, thetas, n_angles, mask, outs,
+                           out_step, out_frame_stride, angle_stride, out_format);
+}
+extern "C" int cvs_g4_steer_bank_host(cvs_g4* h, const void* in, int in_is_u8, int n, int rows, int cols, size_t in_step, size_t in_frame_stride,
+                                      const float* thetas, int n_angles, unsigned mask, void* const* outs, size_t out_step, size_t out_frame_stride,
+                                      size_t angle_stride, int out_format)
+{
+    return steer_bank_host(4, reinterpret_cast<Filter*>(h), in, in_is_u8, n, rows, cols, in_step, in_frame_stride, thetas, n_angles, mask, outs,
+                           out_step, out_frame_stride, angle_stride, out_format);
 }
 
 extern "C" int cvs_to_u8_dev(int device, const float* src, int n, int rows, int cols, size_t pitch, size_t frame_stride, float gain, uint8_t* dst,

@@ -320,6 +320,39 @@ CVS_API int cvs_g2_steer_bank_host(cvs_g2* h, const void* in, int in_is_u8, int 
                                    size_t in_frame_stride, const float* thetas, int n_angles, unsigned mask,
                                    void* const* outs, size_t out_step, size_t out_frame_stride, size_t angle_stride,
                                    int out_format);
+/* G4/H4 steering bank: the 11-plane basis is filtered once per pixel and steered to each of `n_angles` scalar angles in the
+ * same launch -- G4 orientation feature banks and steerable-pyramid levels without re-reading the frames or re-running the
+ * basis march, which is the larger part of the work.  Bits of `mask`: per angle any of CVS_G4T, CVS_H4T, CVS_MAG4,
+ * CVS_PHASE4.  Layout as for cvs_g2_steer_bank_dev: angle k of frame f of plane p at
+ * outs[p] + k*angle_stride + f*out_frame_stride + row*out_pitch, either stride order, no two (angle, frame) planes of one
+ * quantity overlapping.
+ * Contract, for fp32 and 8-bit frames and every out_format: for every k, each selected plane equals, bit for bit (NaN
+ * positions included), that plane of
+ *     cvs_g4_run_batch_dev_fmt(h, b', CVS_G4_MASK_STEER, CVS_STEER_SCALAR, thetas[k], ..., out_format)
+ * where b' is the batch with its frames as fp32: b itself for fp32 frames, the 8-bit frames widened to float (values 0..255,
+ * no scaling) for 8-bit frames.  (With fp32 planes the single-angle call on 8-bit frames itself runs a kernel whose taps are
+ * not prescaled, so its last bits differ from the widened-frames call; the bank follows the widened frames, as the host-buffer
+ * 8-bit calls do.)
+ * No theta_d / strength: the steer@scalar kernels fold the binomial steering factors into the column taps, so the basis
+ * values they steer are not the plain ones the G4 orientation forms need.  Callers who want CVS_G4_THETA / CVS_G4_STRENGTH
+ * make one cvs_g4_run_batch_dev_fmt call for them.
+ * The band fields of `b` and next_level are honoured as in cvs_g4_run_batch_dev.  Argument errors are CVS_ERR_INVALID_ARG
+ * before the handle is looked at and before any CUDA call: n_angles outside [1, CVS_BANK_MAX_ANGLES] or null thetas, mask
+ * bits outside CVS_G4_BANK_PLANES or none, a null selected plane, an unknown out_format and the 16-bit layout rules of the
+ * _fmt calls (angle_stride included), overlapping planes, and (host call) in_step below cols times the element size; so is a
+ * G2 handle.
+ * Speed: with the default width and taps, TMA-eligible frames and planes, pitch and strides aligned to the element size, the
+ * whole batch is one fused launch (cvs_g2_last_launch on the G4 handle: g4_bank/...).  Anything else widens 8-bit frames into
+ * stream-ordered scratch and runs the calls the contract names, one per angle, with unselected quantities in stream-ordered
+ * scratch (bank-fallback:<the per-angle kernel>). */
+#define CVS_G4_BANK_PLANES CVS_G4_MASK_STEER /* per angle: G4T, H4T, MAG4, PHASE4 */
+CVS_API int cvs_g4_steer_bank_dev(cvs_g4* h, const cvs_batch* b, const float* thetas /* host, n_angles */, int n_angles, unsigned mask,
+                                  void* const* outs, size_t angle_stride, void* stream, int out_format);
+/* Host-buffer twin (the pipeline of cvs_g2_steer_bank_host): in_is_u8 selects 8-bit frames, else fp32. */
+CVS_API int cvs_g4_steer_bank_host(cvs_g4* h, const void* in, int in_is_u8, int n, int rows, int cols, size_t in_step,
+                                   size_t in_frame_stride, const float* thetas, int n_angles, unsigned mask,
+                                   void* const* outs, size_t out_step, size_t out_frame_stride, size_t angle_stride,
+                                   int out_format);
 
 /* ---- the callers' 8-bit post-processing (reference example/steer.cpp:92-104, test/test.cpp:93-95), on the device ----
  * gain > 0: Mat::convertTo(CV_8UC1, gain); gain <= 0: cv::normalize(src, dst, 0, 255, NORM_MINMAX, CV_8UC1), per frame. */
